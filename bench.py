@@ -13,17 +13,28 @@ Arms
   default            our CUDA engine through the C ABI of libconcentus_b200.so
                        value : packets and PCM resident in HBM (opus_decode_span_device / opus_encode_span_device)
                        e2e   : pinned host buffers in and out through opus_decode_span / opus_encode_span (H2D + D2H inside the timing)
-  --impl reference   the UNMODIFIED opus-fix C build (oracle/_ref), one stream per thread on all host cores, on a bounded sample
-                     of the same workload.
+  --impl reference   the UNMODIFIED opus-fix C build (oracle/_ref, built by `make -C oracle REF=<opus-fix source tree>`), one
+                     stream per thread on all host cores, on a bounded sample of the same workload.  The same build gives the
+                     "cpu_baseline" objects of the default arm; without it they are null.
 
 Signals (BASELINE.md section 3): stream s plays generate_music with seed 13371337 + s (opus-fix/tests/test_opus_encode.c:59-90);
 every eighth stream instead plays the reference's own parity input `48Khz Stereo.raw` (tests/golden/48Khz_Stereo.raw), cyclically
 shifted by a per-stream offset.  Every stream has `--unique` seconds of its own signal, repeated to the workload's length (the decode
 input is the oracle's encoding of those seconds, its packets repeated: the decoder sees a splice every `--unique` seconds, which is
 as valid a packet sequence as any).  Clicks are added to a quarter of the music streams so that transients / short MDCTs occur.
+The oracle is tests/oracle_lib.py.  The reference's results are stored only for the test suite's inputs, so here the oracle is the
+host simulation of the codec headers, unchecked (pin=False): the parity passes compare the CUDA build with a host build of the same
+headers, and the decode input is coded by the build's own encoder headers.  The result line carries a digest of each decode
+workload's packets ("input_digest"), so runs of two builds can confirm that they decoded the same input.
+
+--dump-outputs DIR writes, after the timed steps, what the timed calls of each workload returned in their last step (PCM and
+return codes of the decode calls, packets and lengths of the encode calls) as DIR/<name>.npy: a fixed, seeded sample of 32 streams
+x 50 frames per workload (float32, plus float64 indices of the sample; at most 42 MB in all, whatever the workload's size), so that
+two builds can be compared output for output.
 """
 import argparse
 import ctypes as C
+import hashlib
 import json
 import os
 import subprocess
@@ -57,7 +68,6 @@ def stream_signals(first, count, seconds, threads):
     n_s = seconds * FS
     out = np.zeros((count, n_s, CH), dtype=np.int16)
     raw = np.fromfile(RAW_FIXTURE, dtype="<i2").reshape(-1, CH) if os.path.exists(RAW_FIXTURE) else None
-    lib = O.ref()
 
     def work(k):
         s = first + k
@@ -68,7 +78,7 @@ def stream_signals(first, count, seconds, threads):
             if len(seg) < n_s:
                 out[k, len(seg):] = np.resize(seg, (n_s - len(seg), CH))
         else:
-            lib.ref_generate_music(O.ptr(out[k]), n_s, (13371337 + s) & 0xFFFFFFFF)
+            out[k] = O.generate_music(n_s, (13371337 + s) & 0xFFFFFFFF)
             if s % 4 == 1:   # clicks: drive the transient detector / short blocks / anti-collapse
                 rs = np.random.RandomState(s)
                 x = out[k].astype(np.int32) // 2
@@ -94,13 +104,10 @@ def oracle_encode(pcm, bitrates, vbr, cvbr, threads, stride):
     vbr = np.broadcast_to(np.asarray(vbr), (n,))
     cvbr = np.broadcast_to(np.asarray(cvbr), (n,))
     keys = sorted(set(zip(bitrates.tolist(), vbr.tolist(), cvbr.tolist())))
-    for (br, v, cv) in keys:   # the MT harness takes one setting per call
+    for (br, v, cv) in keys:   # one setting per call
         idx = np.nonzero((bitrates == br) & (vbr == v) & (cvbr == cv))[0]
-        sub = np.ascontiguousarray(pcm[idx])
-        o = np.zeros((len(idx), F, stride), dtype=np.uint8)
-        l = np.zeros((len(idx), F), dtype=np.int32)
-        cfg = O.RefEncCfg(O.OPUS_APPLICATION_RESTRICTED_LOWDELAY, int(br), int(v), int(cv), 10, stride, 0, 0)
-        O.ref().ref_encode_streams_mt(len(idx), F, threads, O.ptr(sub), FRAME, CH, FS, C.byref(cfg), O.ptr(o), stride, O.ptr(l), None)
+        o, l, _ = O.encode_streams(np.ascontiguousarray(pcm[idx]), FRAME, int(br), threads, vbr=int(v), cvbr=int(cv), complexity=10,
+                                   max_bytes=stride, stride=stride, pin=False)
         out[idx] = o
         lens[idx] = l
     assert (lens > 2).all()
@@ -254,6 +261,21 @@ def shard_range(n, rank, world):
 # ------------------------------------------------------------------------------------------------------------------------------
 # the reference arm
 # ------------------------------------------------------------------------------------------------------------------------------
+def ref_lib(name="libopus_ref.so"):
+    """oracle/_ref/<name>: the unmodified opus-fix build with oracle/ref_harness.c's thread pool; None when it was not built."""
+    p = os.path.join(ROOT, "oracle", "_ref", name)
+    if not os.path.exists(p):
+        return None
+    lib = C.CDLL(p)
+    lib.ref_decode_streams_mt.restype = C.c_double
+    lib.ref_decode_streams_mt.argtypes = [C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p,
+                                          C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]
+    lib.ref_encode_streams_mt.restype = C.c_double
+    lib.ref_encode_streams_mt.argtypes = [C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_int, C.c_int, C.c_int,
+                                          C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p]
+    return lib
+
+
 def decode_input(n, seconds, unique, threads):
     """Packets of the first n streams of the decode workload: (blob, offs, lens, F)."""
     pcm = stream_signals(0, n, unique, threads)
@@ -269,7 +291,7 @@ def decode_input(n, seconds, unique, threads):
 def reference_decode(n, seconds, unique, threads, lib=None, inp=None):
     """The unmodified opus-fix decoder on the first n streams of the decode workload, one stream per thread.  (x realtime, wall s)"""
     import oracle_lib as O
-    lib = lib or O.ref()
+    lib = lib or ref_lib()
     blob, offs, l2, F = inp if inp is not None else decode_input(n, seconds, unique, threads)
     t = lib.ref_decode_streams_mt(n, F, threads, O.ptr(blob), O.ptr(offs), O.ptr(l2), FRAME, CH, FS, None, None, None)
     return n * seconds / t, t
@@ -277,7 +299,7 @@ def reference_decode(n, seconds, unique, threads, lib=None, inp=None):
 
 def reference_encode(n, seconds, unique, threads, lib=None):
     import oracle_lib as O
-    lib = lib or O.ref()
+    lib = lib or ref_lib()
     u = min(unique, seconds)
     pcm = stream_signals(0, n, u, threads)
     reps = (seconds + u - 1) // u
@@ -294,20 +316,13 @@ def reference_encode(n, seconds, unique, threads, lib=None):
 def o3_lib():
     """oracle/_ref/libopus_ref_o3.so: the same unmodified sources at -O3 -march=x86-64-v3 (BASELINE.md section 3: 'so the comparison
     is not against a handicapped baseline'); None when it was not built."""
-    p = os.path.join(ROOT, "oracle", "_ref", "libopus_ref_o3.so")
-    if not os.path.exists(p):
-        return None
-    import oracle_lib as O
-    lib = C.CDLL(p)
-    lib.ref_decode_streams_mt.restype = C.c_double
-    lib.ref_decode_streams_mt.argtypes = O.ref().ref_decode_streams_mt.argtypes
-    lib.ref_encode_streams_mt.restype = C.c_double
-    lib.ref_encode_streams_mt.argtypes = O.ref().ref_encode_streams_mt.argtypes
-    return lib
+    return ref_lib("libopus_ref_o3.so")
 
 
 def cpu_baselines(kind, n, seconds, unique, cores):
-    """The reference on the host cores: -O2 as shipped, and -O3 -march=x86-64-v3 when built."""
+    """The reference on the host cores: -O2 as shipped, and -O3 -march=x86-64-v3 when built; None without the reference build."""
+    if ref_lib() is None:
+        return None
     fn = reference_decode if kind == "decode" else reference_encode
     v, t = fn(n, seconds, unique, cores)
     out = {"value": v, "unit": "x realtime", "cores": cores, "kind": "reference",
@@ -322,6 +337,8 @@ def cpu_baselines(kind, n, seconds, unique, cores):
 def run_reference(args, rank, world):
     if rank != 0:
         return
+    if ref_lib() is None:
+        raise SystemExit("bench.py --impl reference: oracle/_ref/libopus_ref.so not built (make -C oracle REF=<opus-fix source tree>)")
     cores = os.cpu_count() or 1
     n = min(args.streams, max(cores * 4, 16))
     sec = min(args.seconds, 30)
@@ -371,6 +388,48 @@ def barrier(E):
         E.dist.barrier()
 
 
+DUMP_STREAMS, DUMP_FRAMES, DUMP_CAP = 32, 50, 64 << 20
+
+
+def dump_window(S, F):
+    """The fixed sample --dump-outputs writes: DUMP_STREAMS of the S streams and a window of DUMP_FRAMES of the F frames, seeded,
+    so that its size does not grow with the workload (at most 12.3 MB of PCM or 8.2 MB of packets per workload)."""
+    pick = np.sort(np.random.RandomState(1234).choice(S, min(DUMP_STREAMS, S), replace=False))
+    nf = min(DUMP_FRAMES, F)
+    f0 = int(np.random.RandomState(1235).randint(0, F - nf + 1))
+    return pick, f0, nf
+
+
+def dump_pcm(E, name, d_pcm, d_ret, S, F):
+    """PCM [k, nf, FRAME*CH] and return codes [k, nf] of the sampled streams over the sampled frames."""
+    pick, f0, nf = dump_window(S, F)
+    sel = E.torch.from_numpy(pick).to(E.dev)
+    E.dump[name + "_pcm"] = d_pcm.view(S, F, FRAME * CH)[sel, f0:f0 + nf].cpu().numpy().astype(np.float32)
+    E.dump[name + "_ret"] = d_ret.view(S, F)[sel, f0:f0 + nf].cpu().numpy().astype(np.float32)
+    E.dump[name + "_window"] = np.concatenate([pick, [f0, nf]]).astype(np.float64)   # stream indices, first frame, frame count
+
+
+def dump_packets(E, name, d_data, d_ret, S, F, stride):
+    """Packet bytes of the sampled streams over the sampled frames (concatenated in stream / frame order) and their lengths [k, nf]."""
+    pick, f0, nf = dump_window(S, F)
+    sel = E.torch.from_numpy(pick).to(E.dev)
+    rows = d_data.view(S, F, stride)[sel, f0:f0 + nf].cpu().numpy()
+    lens = d_ret.view(S, F)[sel, f0:f0 + nf].cpu().numpy()
+    E.dump[name + "_packets"] = np.concatenate([rows[k, f, :max(int(lens[k, f]), 0)] for k in range(len(pick)) for f in range(nf)]).astype(np.float32)
+    E.dump[name + "_lens"] = lens.astype(np.float32)
+    E.dump[name + "_window"] = np.concatenate([pick, [f0, nf]]).astype(np.float64)
+
+
+def input_digest(pk, lens):
+    """Digest of a decode workload's packets (the oracle's encoding of its signals), so that runs can confirm identical inputs."""
+    h = hashlib.blake2b(digest_size=8)
+    for s in range(pk.shape[0]):
+        for f in range(pk.shape[1]):
+            h.update(pk[s, f, :max(int(lens[s, f]), 0)].tobytes())
+    h.update(np.ascontiguousarray(lens, dtype=np.int32).tobytes())
+    return h.hexdigest()
+
+
 def F_chunk(F):
     for c in (1000, 750, 500, 250, 200, 100, 50, 25, 10, 5, 1):   # packets per e2e call: several pipeline chunks per call
         if F % c == 0:
@@ -387,6 +446,7 @@ def bench_decode(E, args):
     pcm = stream_signals(first, S, args.unique, E.threads)
     pk, lens_u = oracle_encode(pcm, BITRATE, 0, 0, E.threads, 256)
     del pcm
+    digest = input_digest(pk, lens_u)
     plen = int(lens_u[0, 0])
     assert (lens_u == plen).all(), "CBR packets expected"
     Fu = lens_u.shape[1]
@@ -416,7 +476,6 @@ def bench_decode(E, args):
     for _ in range(args.warmup):
         step_value(dec.handles)
     barrier(E)
-    assert bool((d_ret == FRAME).all().item()), "decode returned errors"
     L.opus_b200_stage_times(None, None, 1)
     sampler = ClockSampler(E.local)
     sampler.start()
@@ -429,6 +488,9 @@ def bench_decode(E, args):
     barrier(E)
     ms = all_max(E, e0.elapsed_time(e1))
     clocks = sampler.stop()
+    assert bool((d_ret == FRAME).all().item()), "decode returned errors"
+    if args.dump_outputs:
+        dump_pcm(E, "decode", d_pcm, d_ret, S, F)
     launches = int(L.opus_b200_kernel_launches() - launches0)
     stage_ms = (C.c_double * 3)()
     stage_n = (C.c_longlong * 3)()
@@ -473,16 +535,13 @@ def bench_decode(E, args):
         blob_sel = np.ascontiguousarray(np.tile(pk[pick][:, :, :plen], (1, (F + Fu - 1) // Fu, 1))[:, :F]).reshape(-1)
         o2 = np.arange(nsel * F, dtype=np.int64) * plen
         l2 = np.full(nsel * F, plen, dtype=np.int32)
-        rp = np.zeros((nsel * F * FRAME, CH), dtype=np.int16)
-        rr = np.zeros(nsel * F, dtype=np.uint32)
-        rret = np.zeros(nsel * F, dtype=np.int32)
-        O.ref().ref_decode_streams_mt(nsel, F, E.threads, O.ptr(blob_sel), O.ptr(o2), O.ptr(l2), FRAME, CH, FS, O.ptr(rp), O.ptr(rr), O.ptr(rret))
+        rp, rr, rret = O.decode_streams(nsel, F, E.threads, blob_sel, o2, l2, FRAME, CH, FS, pin=False)
         rp = rp.reshape(nsel, -1)
         bad = [int(s) for k, s in enumerate(pick)
                if not (np.array_equal(rp[k], rows[k]) and int(rr[(k + 1) * F - 1]) == int(fr[s]) and (rret[k * F:(k + 1) * F] == FRAME).all())]
         decp.close()
         parity = {"streams_checked": nsel, "packets_each": int(F), "mismatching_streams": bad,
-                  "against": "oracle/_ref (unmodified opus-fix), fresh state, PCM sample-for-sample + final range"}
+                  "against": "the host simulation of the same codec headers (tests/oracle_lib.py, pin=False), fresh state, PCM sample-for-sample + final range"}
         assert not bad, "decode parity failed at bench size: streams %s" % bad
 
     # ---- e2e: host buffers through opus_decode_span (H2D + kernels + D2H per call) ----
@@ -527,7 +586,8 @@ def bench_decode(E, args):
     dec.close()
     del d_blob
     torch.cuda.empty_cache()
-    return {"value": value, "ms": ms, "clocks": clocks, "launches": launches, "roofline": roofline, "parity": parity, "e2e": e2e, "cpu": cpu}
+    return {"value": value, "ms": ms, "clocks": clocks, "launches": launches, "roofline": roofline, "parity": parity, "e2e": e2e, "cpu": cpu,
+            "input_digest": digest}
 
 
 def barrier_local(E):
@@ -564,8 +624,6 @@ def bench_encode(E, args):
     for _ in range(args.warmup):
         step_value(enc.handles)
     barrier(E)
-    assert bool((d_ret > 2).all().item()), "encode returned errors"
-    mean_len = float(d_ret.float().mean().item())
     launches0 = L.opus_b200_enc_kernel_launches()
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record(estream)
@@ -575,6 +633,10 @@ def bench_encode(E, args):
     barrier(E)
     ms = all_max(E, e0.elapsed_time(e1))
     launches = int(L.opus_b200_enc_kernel_launches() - launches0)
+    assert bool((d_ret > 2).all().item()), "encode returned errors"
+    mean_len = float(d_ret.float().mean().item())
+    if args.dump_outputs:
+        dump_packets(E, "encode", d_data, d_ret, S, F, stride)
     value = E.world * S * seconds * args.steps / (ms / 1e3)
     pc, lc = C.c_longlong(0), C.c_longlong(0)
     L.opus_b200_enc_path_counts(C.byref(pc), C.byref(lc))
@@ -611,11 +673,7 @@ def bench_encode(E, args):
         src = np.ascontiguousarray(d_pcm[sel].cpu().numpy())
         fr = encp.final_ranges()
         nsel = len(pick)
-        rd = np.zeros((nsel, F, 1276), dtype=np.uint8)
-        rl = np.zeros((nsel, F), dtype=np.int32)
-        rr = np.zeros((nsel, F), dtype=np.uint32)
-        cfg = O.RefEncCfg(O.OPUS_APPLICATION_RESTRICTED_LOWDELAY, ENC_BITRATE, 1, 0, 10, 1276, 0, 0)
-        O.ref().ref_encode_streams_mt(nsel, F, E.threads, O.ptr(src), FRAME, CH, FS, C.byref(cfg), O.ptr(rd), 1276, O.ptr(rl), O.ptr(rr))
+        rd, rl, rr = O.encode_streams(src, FRAME, ENC_BITRATE, E.threads, vbr=1, cvbr=0, complexity=10, max_bytes=1276, stride=1276, pin=False)
         bad = []
         for k, sidx in enumerate(pick):
             ok = np.array_equal(rl[k], got_l[k]) and all(np.array_equal(rd[k, f, :rl[k, f]], got_d[k, f, :rl[k, f]]) for f in range(F)) \
@@ -624,7 +682,7 @@ def bench_encode(E, args):
                 bad.append(int(sidx))
         encp.close()
         parity = {"streams_checked": nsel, "frames_each": int(F), "mismatching_streams": bad,
-                  "against": "oracle/_ref (unmodified opus-fix), fresh state, packets byte-for-byte + final range"}
+                  "against": "the host simulation of the same codec headers (tests/oracle_lib.py, pin=False), fresh state, packets byte-for-byte + final range"}
         assert not bad, "encode parity failed at bench size: streams %s" % bad
         # SURVEY.md 8d.3: the workload must exercise the pre-filter and the transient / short-MDCT paths: shares of the oracle's frames
         pf, tr = celt_header_flags(rd.reshape(-1, 1276), rl.reshape(-1))
@@ -688,6 +746,7 @@ def bench_mixed(E, args):
     vbr_u = rs.randint(2, size=U)
     pcm_u = stream_signals(100000, U, seconds, E.threads)                     # [U, T, CH]
     pk_u, len_u = oracle_encode(pcm_u, br_u, vbr_u, 0, E.threads, 1276)       # [U, F, 1276]
+    digest = input_digest(pk_u, len_u)
     prog = (np.arange(lo, hi) % U)
     rot = ((np.arange(lo, hi) // U) * 7) % F
     fidx = (np.arange(F)[None, :] + rot[:, None]) % F                         # [S, F]
@@ -732,7 +791,7 @@ def bench_mixed(E, args):
         for k, s in enumerate(pick):
             u_ = int(prog[s])
             blob_s = np.ascontiguousarray(pk_u[u_]).reshape(-1)
-            rp, _, rret = O.decode_stream(blob_s, np.arange(F, dtype=np.int64) * 1276, len_u[u_], FRAME, CH)
+            rp, _, rret = O.decode_stream(blob_s, np.arange(F, dtype=np.int64) * 1276, len_u[u_], FRAME, CH, pin=False)
             if not (np.array_equal(rp.reshape(-1), rows[k]) and (rret == FRAME).all()):
                 bad.append(int(lo + s))
         parity = {"decode_streams_checked": len(pick), "decode_mismatching": bad}
@@ -744,6 +803,8 @@ def bench_mixed(E, args):
     e1.record(stream)
     barrier(E)
     dms = all_max(E, e0.elapsed_time(e1))
+    if args.dump_outputs:
+        dump_pcm(E, "mixed_decode", d_pcm, d_ret, S, F)
     dec_value = NT * seconds * args.steps / (dms / 1e3)
     dec.close()
     del d_blob, d_pcm
@@ -785,7 +846,7 @@ def bench_mixed(E, args):
                 bad.append(int(lo + s))
         parity["encode_streams_checked"] = len(pick)
         parity["encode_mismatching"] = bad
-        parity["against"] = "oracle/_ref (unmodified opus-fix): PCM sample-for-sample / packets byte-for-byte, fresh state"
+        parity["against"] = "the host simulation of the same codec headers (tests/oracle_lib.py, pin=False): PCM sample-for-sample / packets byte-for-byte, fresh state"
         assert not bad, "mixed encode parity failed: %s" % bad
     e0.record(estream)
     for _ in range(args.steps):
@@ -793,26 +854,33 @@ def bench_mixed(E, args):
     e1.record(estream)
     barrier(E)
     ems = all_max(E, e0.elapsed_time(e1))
+    if args.dump_outputs:
+        dump_packets(E, "mixed_encode", d_data, d_ret, S, F, stride)
     enc_value = NT * seconds * args.steps / (ems / 1e3)
     enc.close()
     del d_in, d_data
     torch.cuda.empty_cache()
     cpu = None
-    if E.rank == 0 and E.world == 1 and not args.no_cpu:
+    if E.rank == 0 and E.world == 1 and not args.no_cpu and ref_lib() is not None:
         nd = min(U, max(E.cores * 8, 32))
         blob = np.ascontiguousarray(pk_u[:nd]).reshape(-1)
         o2 = np.arange(nd * F, dtype=np.int64) * 1276
         l2 = np.ascontiguousarray(len_u[:nd]).reshape(-1)
-        td = O.ref().ref_decode_streams_mt(nd, F, E.cores, O.ptr(blob), O.ptr(o2), O.ptr(l2), FRAME, CH, FS, None, None, None)
-        t0 = time.perf_counter()
-        oracle_encode(pcm_u[:nd], br_u[:nd], vbr_u[:nd], 0, E.cores, 1276)
-        te = time.perf_counter() - t0
+        td = ref_lib().ref_decode_streams_mt(nd, F, E.cores, O.ptr(blob), O.ptr(o2), O.ptr(l2), FRAME, CH, FS, None, None, None)
+        te = 0.0
+        for (br, v) in sorted(set(zip(br_u[:nd].tolist(), vbr_u[:nd].tolist()))):   # one setting per call
+            idx = np.nonzero((br_u[:nd] == br) & (vbr_u[:nd] == v))[0]
+            cfg = O.RefEncCfg(O.OPUS_APPLICATION_RESTRICTED_LOWDELAY, int(br), int(v), 0, 10, 1276, 0, 0)
+            o = np.zeros((len(idx), F, 1276), dtype=np.uint8)
+            l = np.zeros((len(idx), F), dtype=np.int32)
+            te += ref_lib().ref_encode_streams_mt(len(idx), F, E.cores, O.ptr(np.ascontiguousarray(pcm_u[idx])), FRAME, CH, FS, C.byref(cfg),
+                                                  O.ptr(o), 1276, O.ptr(l), None)
         cpu = {"decode": nd * seconds / td, "encode": nd * seconds / te, "unit": "x realtime", "cores": E.cores, "kind": "reference",
                "sample": "%d of the %d programmes x %d s, opus-fix -O2, one stream per thread" % (nd, U, seconds)}
     return {"metric": "CELT mixed-bitrate decode / encode audio-sec per sec (x realtime), 48k stereo, %d streams" % NT,
             "decode": {"value": dec_value, "unit": "x realtime", "ms_per_step": dms / args.steps},
             "encode": {"value": enc_value, "unit": "x realtime", "ms_per_step": ems / args.steps},
-            "streams_this_rank": int(S), "scaling": "strong", "config": mixed_config(args, E.world), "parity": parity, "cpu_baseline": cpu}
+            "streams_this_rank": int(S), "scaling": "strong", "input_digest": digest, "config": mixed_config(args, E.world), "parity": parity, "cpu_baseline": cpu}
 
 
 def main():
@@ -834,6 +902,7 @@ def main():
     ap.add_argument("--no-encode", action="store_true")
     ap.add_argument("--no-mixed", action="store_true")
     ap.add_argument("--no-parity", action="store_true", help="skip the untimed full-size parity passes against the oracle")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the timed calls returned in their last step to DIR/<name>.npy")
     args = ap.parse_args()
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -860,6 +929,7 @@ def main():
     E.cores = os.cpu_count() or 1
     E.threads = max(1, E.cores // max(world, 1))
     E.peaks = {}
+    E.dump = {}
     try:
         E.peaks = json.load(open(os.path.join(ROOT, "MEASURED_PEAKS.json")))
     except Exception:
@@ -878,8 +948,14 @@ def main():
         line = {"metric": METRIC, "value": d["value"], "unit": "x realtime", "n_gpus": world, "steps": args.steps, "warmup": args.warmup,
                 "ms_per_step": d["ms"] / args.steps, "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "int32",
                 "data": "synthetic", "config": decode_config(args, world), "clocks": d["clocks"], "e2e": d["e2e"], "gpu_launches": int(launches),
-                "roofline": d["roofline"], "cpu_baseline": d["cpu"], "parity": d["parity"], "encode": encode, "mixed": mixed}
+                "roofline": d["roofline"], "cpu_baseline": d["cpu"], "parity": d["parity"], "input_digest": d["input_digest"],
+                "encode": encode, "mixed": mixed}
         print(json.dumps(line), flush=True)
+        if args.dump_outputs:
+            assert sum(a.nbytes for a in E.dump.values()) <= DUMP_CAP, "--dump-outputs: sample larger than 64 MB"
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            for name, a in E.dump.items():
+                np.save(os.path.join(args.dump_outputs, name + ".npy"), a)
     if E.dist is not None:
         E.dist.destroy_process_group()
 

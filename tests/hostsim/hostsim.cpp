@@ -11,6 +11,31 @@
 
 extern "C" {
 
+// The tests' music signal (tests/oracle_lib.py generate_music), the same function as ref_generate_music in oracle/ref_harness.c:
+// opus-fix/tests/test_opus_encode.c:59-90 driven by the MWC generator of tests/test_opus_common.h:55-62 with an explicit seed.
+void hostsim_generate_music(int16_t *buf, int32_t len, uint32_t seed) {
+    uint32_t Rz = seed, Rw = seed;
+    int32_t a1 = 0, b1 = 0, a2 = 0, b2 = 0, c1 = 0, c2 = 0, d1 = 0, d2 = 0, j = 0;
+    for (int32_t i = 0; i < len; i++) {
+        uint32_t r;
+        int32_t v1, v2;
+        v1 = v2 = (((j * ((j >> 12) ^ ((j >> 10 | j >> 12) & 26 & j >> 7))) & 128) + 128) << 15;
+        Rz = 36969 * (Rz & 65535) + (Rz >> 16); Rw = 18000 * (Rw & 65535) + (Rw >> 16);
+        r = (Rz << 16) + Rw; v1 += r & 65535; v1 -= r >> 16;
+        Rz = 36969 * (Rz & 65535) + (Rz >> 16); Rw = 18000 * (Rw & 65535) + (Rw >> 16);
+        r = (Rz << 16) + Rw; v2 += r & 65535; v2 -= r >> 16;
+        b1 = v1 - a1 + ((b1 * 61 + 32) >> 6); a1 = v1;
+        b2 = v2 - a2 + ((b2 * 61 + 32) >> 6); a2 = v2;
+        c1 = (30 * (c1 + b1 + d1) + 32) >> 6; d1 = b1;
+        c2 = (30 * (c2 + b2 + d2) + 32) >> 6; d2 = b2;
+        v1 = (c1 + 128) >> 8;
+        v2 = (c2 + 128) >> 8;
+        buf[i * 2] = v1 > 32767 ? 32767 : (v1 < -32768 ? -32768 : v1);
+        buf[i * 2 + 1] = v2 > 32767 ? 32767 : (v2 < -32768 ? -32768 : v2);
+        if (i % 6 == 0) j++;
+    }
+}
+
 int hostsim_dec_state_size(void) { return (int)sizeof(CbDecState); }
 
 // Decode F packets of one stream (packed layout).  cap = pcm capacity per packet (samples per channel).

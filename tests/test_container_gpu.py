@@ -1,32 +1,42 @@
-"""GPU: batch file coding through the `.bit` container (concentus_b200/bitfile.py, SURVEY.md §8f rank 4), checked by the
-reference's own command-line codec (oracle/_ref/opus_demo, built from the unmodified src/opus_demo.c): it decodes the files our
-CUDA encoder wrote — verifying the stored final range against its decoder on every packet (src/opus_demo.c:806-816) — and our
-CUDA decoder must reproduce its output for files it wrote."""
-import os
-import subprocess
-
+"""GPU: batch file coding through the `.bit` container (concentus_b200/bitfile.py, SURVEY.md §8f rank 4), checked against what
+the reference's own command-line codec (src/opus_demo.c) does with such files: it decodes the files our CUDA encoder wrote —
+verifying the stored final range against its decoder on every packet (src/opus_demo.c:806-816) — and our CUDA decoder must
+reproduce its output for files it wrote.  The reference's side is restated through the oracle (tests/oracle_lib.py)."""
 import numpy as np
 import pytest
 
 import oracle_lib as O
 
 pytestmark = pytest.mark.gpu
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-DEMO = os.path.join(ROOT, "oracle", "_ref", "opus_demo")
 
 
 def _cb():
     import concentus_b200 as cb
     assert cb.lib().opus_b200_init(0) == 0, "CUDA device required: no CPU fallback exists"
-    assert os.path.exists(DEMO), "oracle/_ref/opus_demo missing (built by `make -C oracle` where the reference sources exist)"
     return cb
 
 
-def _demo_decode(bit, ch, out):
-    r = subprocess.run([DEMO, "-d", "48000", str(ch), str(bit), str(out)], capture_output=True, text=True)
-    assert r.returncode == 0, r.stderr[-2000:]
-    assert "Range coder state mismatch" not in r.stderr
-    return np.fromfile(out, dtype="<i2").reshape(-1, ch)
+def _demo_decode(bit, ch, fs):
+    """`opus_demo -d 48000 <ch> <bit> <out>`: every record decoded (length 0 = lost packet), the stored final range checked
+    against the decoder's for every received packet, the samples of every packet written."""
+    from concentus_b200 import bitfile
+    data, offs, lens, ranges = bitfile.read_bit(str(bit))
+    pcm, rng, rets = O.decode_stream(data, offs, lens, fs, ch)
+    assert (rets == fs).all(), rets
+    got = lens > 0
+    assert np.array_equal(rng[got], ranges[got]), "Range coder state mismatch"
+    return pcm
+
+
+def _demo_encode(pcm, ch, fs, br, bit):
+    """`opus_demo -e restricted-lowdelay 48000 <ch> <br> [-framesize <fs>] <raw> <bit>` (VBR, complexity 10): the input is coded
+    in whole frames, zero-padded, with one extra frame when it ends on a frame boundary (src/opus_demo.c:672-690)."""
+    from concentus_b200 import bitfile
+    x = np.zeros(((len(pcm) // fs + 1) * fs, ch), dtype=np.int16)
+    x[:len(pcm)] = pcm
+    d, o, l, r = O.encode_stream(x, fs, br, ch, vbr=1, cvbr=0, complexity=10, max_bytes=1500)
+    d, o = O.pack(d, o, l)
+    bitfile.write_bit(str(bit), d, o, l, r)
 
 
 @pytest.mark.parametrize("ch,fs,br", [(2, 960, 96000), (1, 480, 64000)])
@@ -49,7 +59,7 @@ def test_our_files_decode_in_the_reference_tool(tmp_path, ch, fs, br):
         for f in range(nf[i]):
             assert np.array_equal(data[offs[f]:offs[f] + lens[f]], rd[ro[f]:ro[f] + rl[f]]), (i, f)
         # the reference tool accepts the file (range check on every packet) and decodes it to what our decoder gives
-        ref = _demo_decode(paths[i], ch, tmp_path / ("s%d.raw" % i))
+        ref = _demo_decode(paths[i], ch, fs)
         assert ref.shape == ours[i].shape and np.array_equal(ref, ours[i]), i
 
 
@@ -60,11 +70,8 @@ def test_reference_files_with_loss_decode_like_the_reference_tool(tmp_path):
     paths = []
     for i, (nsamp, br) in enumerate(((48000, 64000), (30000, 128000), (19200, 32000))):
         pcm = O.test_signal(nsamp, ch, 310 + i, ("music", "tone", "noise")[i])
-        raw = tmp_path / ("r%d.raw" % i)
-        pcm.astype("<i2").tofile(raw)
         bit = tmp_path / ("r%d.bit" % i)
-        r = subprocess.run([DEMO, "-e", "restricted-lowdelay", "48000", str(ch), str(br), str(raw), str(bit)], capture_output=True, text=True)
-        assert r.returncode == 0, r.stderr[-2000:]
+        _demo_encode(pcm, ch, fs, br, bit)
         if i == 1:   # knock packets out of the second file: length-0 records are lost packets (src/opus_demo.c:763)
             d, o, l, rg = bitfile.read_bit(str(bit))
             l = l.copy()
@@ -74,5 +81,5 @@ def test_reference_files_with_loss_decode_like_the_reference_tool(tmp_path):
         paths.append(str(bit))
     ours = bitfile.decode_files(paths, 48000, ch, fs)
     for i, p in enumerate(paths):
-        ref = _demo_decode(p, ch, tmp_path / ("o%d.raw" % i))
+        ref = _demo_decode(p, ch, fs)
         assert ref.shape == ours[i].shape and np.array_equal(ref, ours[i]), i

@@ -1,8 +1,10 @@
-"""CPU-side tests (no GPU needed): the oracle is pinned against the reference's own golden values and our committed
-fixtures; the host simulation of the kernel headers (tests/hostsim, a test tool) is diffed against both; the C ABI
+"""CPU-side tests (no GPU needed): the oracle (tests/oracle_lib.py) is pinned against the reference's own golden values and our
+committed fixtures; the host simulation of the kernel headers (tests/hostsim, a test tool) is diffed against both; the C ABI
 library loads, exports every symbol include/*.h declares and refuses to run without a CUDA device."""
 import ctypes as C
 import glob
+import hashlib
+import json
 import os
 import re
 import struct
@@ -18,8 +20,9 @@ import oracle_lib as O
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 GOLDEN = sorted(p for p in glob.glob(os.path.join(ROOT, "tests", "golden", "*.npz")) if not os.path.basename(p).startswith("enc_"))
 GOLDEN_ENC = sorted(glob.glob(os.path.join(ROOT, "tests", "golden", "enc_*.npz")))
-HAVE_REF = os.path.exists(O.REF_SO) or os.path.isdir("/root/reference/opus-fix")
-needs_ref = pytest.mark.skipif(not HAVE_REF, reason="oracle/_ref not built and reference sources absent")
+# What the reference's repacketizer / opus_packet_pad returned in the comparisons below (return codes and output bytes, in call
+# order), as a digest: recorded when these tests last ran against the reference build, whose results ours matched call for call.
+REF_RESULTS = os.path.join(ROOT, "tests", "golden", "reference_results.json")
 
 
 def _hostsim():
@@ -50,6 +53,23 @@ def _hostsim_encode(hs, pcm, fs, br, ch, vbr, cvbr, cx, application=O.OPUS_APPLI
     cfg = np.array([application, br, vbr, cvbr, cx, max_bytes, 0, 0], dtype=np.int32)
     hs.hostsim_encode_stream(O.ptr(pcm), F, fs, ch, 48000, O.ptr(cfg), O.ptr(out), 1276, O.ptr(lens), O.ptr(rng))
     return out, lens, rng
+
+
+class _RefResults:
+    """The results the reference returned in one of the comparisons below, in call order, checked as one digest (REF_RESULTS)."""
+
+    def __init__(self, name):
+        self.name = name
+        self.h = hashlib.blake2b(digest_size=16)
+
+    def add(self, *vals):
+        for v in vals:
+            self.h.update(np.ascontiguousarray(v).tobytes() if isinstance(v, np.ndarray) else repr(int(v)).encode())
+            self.h.update(b"|")
+
+    def check(self):
+        want = json.load(open(REF_RESULTS))[self.name]
+        assert self.h.hexdigest() == want, "%s: results differ from the reference's (digest %s)" % (self.name, self.h.hexdigest())
 
 
 def _same_packets(g_data, g_offs, g_lens, out, lens):
@@ -89,7 +109,6 @@ def cres_packets(cfg):
     return data, np.arange(65536, dtype=np.int64) * 4, np.full(65536, 4, dtype=np.int32)
 
 
-@needs_ref
 @pytest.mark.parametrize("path", GOLDEN, ids=[os.path.basename(p)[:-4] for p in GOLDEN])
 def test_oracle_reproduces_golden(path):
     g = np.load(path)
@@ -99,7 +118,6 @@ def test_oracle_reproduces_golden(path):
     assert np.array_equal(g["enc_ranges"], g["dec_ranges"])
 
 
-@needs_ref
 @pytest.mark.parametrize("cfg", [16, 28])
 def test_oracle_pinned_by_reference_cres_kat(cfg):
     data, offs, lens = cres_packets(cfg)
@@ -123,7 +141,6 @@ def test_hostsim_cres_kat(cfg):
     assert int(rng.astype(np.uint64).sum() & 0xFFFFFFFF) == CRES[cfg]
 
 
-@needs_ref
 def test_hostsim_vs_oracle_mini_sweep():
     hs = _hostsim()
     seed = 77
@@ -141,7 +158,6 @@ def test_hostsim_vs_oracle_mini_sweep():
 
 # ---- encoder --------------------------------------------------------------------------------------------------------
 
-@needs_ref
 @pytest.mark.parametrize("path", GOLDEN_ENC, ids=[os.path.basename(p)[:-4] for p in GOLDEN_ENC])
 def test_oracle_reproduces_encoder_golden(path):
     g = np.load(path)
@@ -163,7 +179,6 @@ def test_hostsim_encoder_matches_golden(path):
     assert np.array_equal(rng, g["enc_ranges"])
 
 
-@needs_ref
 def test_hostsim_encoder_vs_oracle_mini_sweep():
     """BASELINE configs[3] in miniature: frame size x channels x bitrate x CBR/VBR/CVBR x complexity x signal kind."""
     hs = _hostsim()
@@ -190,7 +205,6 @@ def _hostsim_encode_pipe(hs, pcm, fs, br, ch, vbr, cvbr, cx, Fs=48000, max_bytes
     return rc, out, lens, rng
 
 
-@needs_ref
 @pytest.mark.parametrize("band_mode", [2, 1, 0], ids=["inline_walk", "split_chains", "one_stage"])
 def test_hostsim_encoder_pipeline_vs_oracle_mini_sweep(band_mode):
     """The pipeline's slicing of the frame (prepass / front end / head / comb / transform / decide / bands) against the oracle:
@@ -211,7 +225,6 @@ def test_hostsim_encoder_pipeline_vs_oracle_mini_sweep(band_mode):
     hs.hostsim_set_band_mode(2)
 
 
-@needs_ref
 def test_hostsim_encoder_pipeline_long_and_api_rates():
     hs = _hostsim()
     hs.hostsim_set_band_mode(2)
@@ -238,7 +251,6 @@ def test_hostsim_encoder_pipeline_long_and_api_rates():
         assert rc == 0 and _same_packets(d, o, l, out, lens) and np.array_equal(r, rng), (ch, fs, br, maxb)
 
 
-@needs_ref
 def test_hostsim_encoder_long_vbr_and_audio_application():
     """The VBR controller settles over ~970 frames (vbr_count); OPUS_APPLICATION_AUDIO adds 4 ms of delay compensation."""
     hs = _hostsim()
@@ -254,7 +266,6 @@ def test_hostsim_encoder_long_vbr_and_audio_application():
         assert _same_packets(d, o, l, out, lens) and np.array_equal(r, rng), (ch, fs, br)
 
 
-@needs_ref
 def test_hostsim_encoder_other_api_rates():
     """Encoder at 8/12/16/24 kHz API rates, both applications, every frame size."""
     hs = _hostsim()
@@ -279,7 +290,6 @@ def test_hostsim_encoder_other_api_rates():
                 assert _same_packets(d, o, l, out, lens) and np.array_equal(r, rng), (Fs, ch, ms, br, app)
 
 
-@needs_ref
 def test_hostsim_encoder_long_frames():
     """40 / 60 ms frames through the repacketizer path, VBR and padded CBR, with and without a tight max_data_bytes."""
     hs = _hostsim()
@@ -302,7 +312,6 @@ def test_hostsim_encoder_long_frames():
                     assert _same_packets(d, o, l, out, lens) and np.array_equal(r, rng), (Fs, ch, ms, br, maxb)
 
 
-@needs_ref
 def test_hostsim_encoder_ctl_fuzz_vs_oracle():
     """Random ctl changes between frames (bitrate incl. AUTO/MAX, VBR / CVBR, complexity, forced channels, bandwidth caps, loss %,
     LSB depth, prediction, signal type, RESET_STATE) — the reference's own fuzz shape (tests/test_opus_encode.c:236-330), every
@@ -361,18 +370,16 @@ def test_encoder_host_api_ctl_and_padding():
     # padding: a code-0 packet grown to every size up to +600 bytes, and back
     pk = np.zeros(1276, dtype=np.uint8)
     pk[:40] = np.arange(40) + 0xF8
+    ref = _RefResults("opus_packet_pad_code0")
     for new_len in (40, 41, 42, 100, 295, 296, 297, 640):
         a = pk.copy()
         assert L.opus_packet_pad(O.ptr(a), 40, new_len) == 0
-        if HAVE_REF:
-            b = pk.copy()
-            assert O.ref().opus_packet_pad(O.ptr(b), 40, new_len) == 0
-            assert np.array_equal(a[:new_len], b[:new_len]), new_len
+        ref.add(a[:new_len])
         assert L.opus_packet_unpad(O.ptr(a), new_len) == 40 and np.array_equal(a[:40], pk[:40])
     assert L.opus_packet_pad(O.ptr(pk), 40, 39) == cb.OPUS_BAD_ARG
+    ref.check()                                    # the padded packets are the reference's, byte for byte
 
 
-@needs_ref
 @pytest.mark.parametrize("pattern", ["single", "burst", "random", "toc_only", "start_lost"])
 def test_hostsim_packet_loss_concealment_vs_oracle(pattern):
     """celt_decode_lost (pitch-based and, after 5 losses, noise-based) through the host simulation of the stage-B code."""
@@ -414,12 +421,11 @@ def test_hostsim_garbage_packets_do_not_crash_and_match_oracle():
         data[offs[f]] = 0x80 | (rs.randint(0, 16) << 3) | (rs.randint(0, 2) << 2)
     hp, hr, hret = _hostsim_decode(hs, data, offs, lens, 960, 2)
     assert ((hret > 0) | (hret == -3)).all()    # garbage may overrun its bit budget: OPUS_INTERNAL_ERROR like the reference
-    if HAVE_REF:
-        rp, rr, rret = O.decode_stream(data, offs, lens, 960, 2)
-        assert np.array_equal(rret, hret) and np.array_equal(rr, hr)
-        for f in range(F):
-            n = max(int(hret[f]), 0)
-            assert np.array_equal(rp[f * 960:f * 960 + n], hp[f * 960:f * 960 + n]), f
+    rp, rr, rret = O.decode_stream(data, offs, lens, 960, 2)
+    assert np.array_equal(rret, hret) and np.array_equal(rr, hr)
+    for f in range(F):
+        n = max(int(hret[f]), 0)
+        assert np.array_equal(rp[f * 960:f * 960 + n], hp[f * 960:f * 960 + n]), f
 
 
 def _declared_symbols():
@@ -519,26 +525,20 @@ def test_stream_sharding_world_size_2_gloo():
 
 # ---- the .bit container (SURVEY.md §8f rank 4): pinned on files written by the reference's own opus_demo -----------------------
 
-def _opus_demo():
-    exe = os.path.join(ROOT, "oracle", "_ref", "opus_demo")
-    O.ref()   # builds oracle/_ref (library and opus_demo) when the reference sources are present
-    assert os.path.exists(exe), "oracle/_ref/opus_demo missing: run `make -C oracle` where /root/reference exists"
-    return exe
+def _opus_demo_file(ch, fs, br):
+    """tests/golden/opus_demo_*.bit: the file `opus_demo -e restricted-lowdelay 48000 <ch> <br> -framesize <ms>` of the reference
+    wrote for test_signal(48000, ch, 77 + ch, "music")."""
+    ms = {120: "2.5", 240: "5", 480: "10", 960: "20"}[fs]
+    return os.path.join(ROOT, "tests", "golden", "opus_demo_%dch_%sms_%dk.bit" % (ch, ms, br // 1000))
 
 
 @pytest.mark.parametrize("ch,fs,br", [(2, 960, 64000), (1, 480, 48000), (2, 120, 128000)])
 def test_bit_container_reads_what_opus_demo_writes(tmp_path, ch, fs, br):
-    """opus_demo -e (src/opus_demo.c:748-760) writes the file; our reader must return exactly the packets and final ranges the
+    """opus_demo -e (src/opus_demo.c:748-760) wrote the file; our reader must return exactly the packets and final ranges the
     oracle's encoder produces for the same input, and our writer must reproduce the file byte for byte."""
     from concentus_b200 import bitfile
     pcm = O.test_signal(48000, ch, 77 + ch, "music")
-    raw = tmp_path / "in.raw"
-    pcm.astype("<i2").tofile(raw)
-    bit = tmp_path / "ref.bit"
-    ms = {120: "2.5", 240: "5", 480: "10", 960: "20"}[fs]
-    r = subprocess.run([_opus_demo(), "-e", "restricted-lowdelay", "48000", str(ch), str(br), "-framesize", ms, str(raw), str(bit)],
-                       capture_output=True, text=True)
-    assert r.returncode == 0, r.stderr[-2000:]
+    bit = _opus_demo_file(ch, fs, br)
     data, offs, lens, ranges = bitfile.read_bit(str(bit))
     # opus_demo codes one extra all-zero frame when the input ends on a frame boundary (src/opus_demo.c:672-690)
     x = np.concatenate([pcm, np.zeros((fs, ch), dtype=np.int16)])
@@ -618,26 +618,25 @@ def test_hostsim_random_wide_sweep():
     assert not bad, bad[:3]
 
 
-@needs_ref
 def test_repacketizer_and_pad_unpad_match_the_reference():
     """opus_repacketizer_* and opus_packet_pad / opus_packet_unpad for packets of every frame-count code (host code of the library,
     opus-fix/src/repacketizer.c:37-273): same return codes and bytes as the reference on random merges, splits and paddings."""
     import concentus_b200 as cb
-    L, R = cb.lib(), O.ref()
-    for lib in (L, R):
-        lib.opus_repacketizer_create.restype = C.c_void_p
-        lib.opus_repacketizer_init.restype = C.c_void_p
-        lib.opus_repacketizer_init.argtypes = [C.c_void_p]
-        lib.opus_repacketizer_destroy.argtypes = [C.c_void_p]
-        lib.opus_repacketizer_cat.argtypes = [C.c_void_p, C.c_void_p, C.c_int32]
-        lib.opus_repacketizer_get_nb_frames.argtypes = [C.c_void_p]
-        lib.opus_repacketizer_out.argtypes = [C.c_void_p, C.c_void_p, C.c_int32]
-        lib.opus_repacketizer_out_range.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_int32]
-        lib.opus_packet_pad.argtypes = [C.c_void_p, C.c_int32, C.c_int32]
-        lib.opus_packet_unpad.argtypes = [C.c_void_p, C.c_int32]
+    L = cb.lib()
+    L.opus_repacketizer_create.restype = C.c_void_p
+    L.opus_repacketizer_init.restype = C.c_void_p
+    L.opus_repacketizer_init.argtypes = [C.c_void_p]
+    L.opus_repacketizer_destroy.argtypes = [C.c_void_p]
+    L.opus_repacketizer_cat.argtypes = [C.c_void_p, C.c_void_p, C.c_int32]
+    L.opus_repacketizer_get_nb_frames.argtypes = [C.c_void_p]
+    L.opus_repacketizer_out.argtypes = [C.c_void_p, C.c_void_p, C.c_int32]
+    L.opus_repacketizer_out_range.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_int32]
+    L.opus_packet_pad.argtypes = [C.c_void_p, C.c_int32, C.c_int32]
+    L.opus_packet_unpad.argtypes = [C.c_void_p, C.c_int32]
     assert L.opus_repacketizer_get_size() > 0
+    ref = _RefResults("repacketizer_pad_unpad")
     rs = np.random.RandomState(5)
-    rp_l, rp_r = L.opus_repacketizer_create(), R.opus_repacketizer_create()
+    rp_l = L.opus_repacketizer_create()
     n_multi = 0
     for trial in range(60):
         fs = (120, 240, 480, 960)[trial % 4]
@@ -650,45 +649,39 @@ def test_repacketizer_and_pad_unpad_match_the_reference():
             pk[3] = np.ascontiguousarray(pk[3][:1])            # a TOC-only packet among them
         if trial % 7 == 6:
             pk[2] = pk[2].copy(); pk[2][0] ^= 0x08             # a packet of another configuration: must be refused
-        L.opus_repacketizer_init(rp_l); R.opus_repacketizer_init(rp_r)
+        L.opus_repacketizer_init(rp_l)
         ncat = int(rs.randint(1, 9))
         for k in range(ncat):
-            a = L.opus_repacketizer_cat(rp_l, O.ptr(pk[k]), len(pk[k]))
-            b = R.opus_repacketizer_cat(rp_r, O.ptr(pk[k]), len(pk[k]))
-            assert a == b, (trial, k, a, b)
+            ref.add(L.opus_repacketizer_cat(rp_l, O.ptr(pk[k]), len(pk[k])))
         nf = L.opus_repacketizer_get_nb_frames(rp_l)
-        assert nf == R.opus_repacketizer_get_nb_frames(rp_r)
+        ref.add(nf)
         for maxlen in (3000, int(rs.randint(1, 600)), 1):
-            ol, orr = np.zeros(3000, dtype=np.uint8), np.zeros(3000, dtype=np.uint8)
+            ol = np.zeros(3000, dtype=np.uint8)
             a = L.opus_repacketizer_out(rp_l, O.ptr(ol), maxlen)
-            b = R.opus_repacketizer_out(rp_r, O.ptr(orr), maxlen)
-            assert a == b and (a < 0 or np.array_equal(ol[:a], orr[:a])), (trial, maxlen, a, b)
+            ref.add(a, ol[:max(a, 0)])
             if nf >= 1:
                 lo = int(rs.randint(0, nf)); hi = int(rs.randint(lo, nf + 2))
                 a = L.opus_repacketizer_out_range(rp_l, lo, hi, O.ptr(ol), maxlen)
-                b = R.opus_repacketizer_out_range(rp_r, lo, hi, O.ptr(orr), maxlen)
-                assert a == b and (a < 0 or np.array_equal(ol[:a], orr[:a])), (trial, lo, hi, maxlen, a, b)
+                ref.add(a, ol[:max(a, 0)])
         # pad / unpad of the merged (multi-frame) packet, in place
         ol = np.zeros(4000, dtype=np.uint8)
         n = L.opus_repacketizer_out(rp_l, O.ptr(ol), 3000)
         if n > 0:
             n_multi += nf > 1
             for new_len in (n, n + 1, n + 2, n + int(rs.randint(3, 700)), n - 1):
-                bl, br = ol.copy(), ol.copy()
+                bl = ol.copy()
                 a = L.opus_packet_pad(O.ptr(bl), n, new_len)
-                b = R.opus_packet_pad(O.ptr(br), n, new_len)
-                assert a == b, (trial, n, new_len, a, b)
+                ref.add(a)
                 if a == 0:
-                    assert np.array_equal(bl[:new_len], br[:new_len]), (trial, n, new_len)
+                    ref.add(bl[:new_len])
                     a = L.opus_packet_unpad(O.ptr(bl), new_len)
-                    b = R.opus_packet_unpad(O.ptr(br), new_len)
-                    assert a == b and np.array_equal(bl[:a], br[:a]), (trial, new_len, a, b)
+                    ref.add(a, bl[:max(a, 0)])
     assert n_multi >= 30
     for bad in (0, -3):
         buf = np.zeros(16, dtype=np.uint8)
-        assert L.opus_packet_pad(O.ptr(buf), bad, 8) == R.opus_packet_pad(O.ptr(buf), bad, 8)
-        assert L.opus_packet_unpad(O.ptr(buf), bad) == R.opus_packet_unpad(O.ptr(buf), bad)
-    L.opus_repacketizer_destroy(rp_l); R.opus_repacketizer_destroy(rp_r)
+        ref.add(L.opus_packet_pad(O.ptr(buf), bad, 8), L.opus_packet_unpad(O.ptr(buf), bad))
+    L.opus_repacketizer_destroy(rp_l)
+    ref.check()
 
 
 def test_public_header_compiles_reference_style_ctl_calls(tmp_path):

@@ -94,10 +94,7 @@ def test_fuzz_million_packets(Fs, channels, cap):
         pcm, rets = dec.decode_span(blob, offs, lens, F, cap)
         fr = dec.final_ranges()
         dec.close()
-        rpcm = np.zeros((n * F * cap, channels), dtype=np.int16)
-        rrng = np.zeros(n * F, dtype=np.uint32)
-        rret = np.zeros(n * F, dtype=np.int32)
-        O.ref().ref_decode_streams_mt(n, F, threads, O.ptr(blob), O.ptr(offs), O.ptr(lens), cap, channels, Fs, O.ptr(rpcm), O.ptr(rrng), O.ptr(rret))
+        rpcm, rrng, rret = O.decode_streams(n, F, threads, blob, offs, lens, cap, channels, Fs=Fs, pin=True)
         bad = np.nonzero(rets != rret)[0]
         assert len(bad) == 0, ("return codes", Fs, r, int(bad[0]) // F, int(bad[0]) % F, int(rets[bad[0]]), int(rret[bad[0]]), int(lens[bad[0]]))
         # decoded samples of every packet that produced any

@@ -2,8 +2,8 @@
 tests/test_opus_decode.c and tests/test_opus_api.c, compiled from the reference's unmodified sources against the reference's
 headers and linked to libconcentus_b200.so by the committed recipe oracle/Makefile (target `b200`; the decode test is restricted
 to the CELT configurations and the API test loses its multistream sections through the committed sed scripts
-oracle/celt_only_decode.sed / oracle/no_multistream_api.sed).  The binaries are built where the reference sources are
-(this container) and travel to the GPU box in oracle/_ref/."""
+oracle/celt_only_decode.sed / oracle/no_multistream_api.sed).  The reference's sources are not part of this repository: the
+binaries exist only where `make -C oracle REF=<opus-fix source tree>` was run, and these tests skip elsewhere."""
 import os
 import subprocess
 
@@ -21,8 +21,7 @@ REF = os.path.join(ROOT, "oracle", "_ref")
 def _need(name):
     p = os.path.join(REF, name)
     if not os.path.exists(p):
-        O.build_ref()
-    assert os.path.exists(p), "%s missing: run `make -C oracle` where /root/reference is present" % name
+        pytest.skip("oracle/_ref/%s not built: needs the reference's sources (make -C oracle REF=<opus-fix source tree>)" % name)
     return p
 
 

@@ -15,7 +15,7 @@ pcm, rets = dec.decode_span(data, offs, lens, F, fs)
 print("rets", rets.reshape(n, F))
 for s in range(n):
     sl = slice(s * F, (s + 1) * F)
-    rp, rr, _ = O.decode_stream(data, offs[sl], lens[sl], fs, 2)
+    rp, rr, _ = O.decode_stream(data, offs[sl], lens[sl], fs, 2, pin=False)
     mine = pcm[s * F * fs:(s + 1) * F * fs]
     bad = np.nonzero((rp.reshape(F, -1) != mine.reshape(F, -1)).any(axis=1))[0]
     print("stream", s, "bad frames", bad)

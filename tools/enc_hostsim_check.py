@@ -27,7 +27,7 @@ def sim_encode(pcm, frame_size, bitrate, channels, vbr=1, cvbr=0, complexity=10,
 
 def compare(kind, channels, frame_size, bitrate, vbr, cvbr, complexity, seconds=2, seed=1234, verbose=True):
     pcm = O.test_signal(48000 * seconds, channels, seed, kind)
-    d, o, l, r = O.encode_stream(pcm, frame_size, bitrate, channels, vbr=vbr, cvbr=cvbr, complexity=complexity)
+    d, o, l, r = O.encode_stream(pcm, frame_size, bitrate, channels, vbr=vbr, cvbr=cvbr, complexity=complexity, pin=False)
     d2, l2, r2, rc = sim_encode(pcm, frame_size, bitrate, channels, vbr=vbr, cvbr=cvbr, complexity=complexity)
     F = len(l)
     bad = -1

@@ -31,7 +31,7 @@ def run(i):
         _hs.hostsim_set_band_mode(2)
     kind, ch, fs, br, (vbr, cvbr), cx = CASES[i]
     x = O.test_signal(int(48000 * SECONDS), ch, 9000 + i, kind)
-    d, o, l, r = O.encode_stream(x, fs, br, ch, vbr=vbr, cvbr=cvbr, complexity=cx, max_bytes=1276)
+    d, o, l, r = O.encode_stream(x, fs, br, ch, vbr=vbr, cvbr=cvbr, complexity=cx, max_bytes=1276, pin=False)
     rc, out, lens, rng = T._hostsim_encode_pipe(_hs, x, fs, br, ch, vbr, cvbr, cx, Fc=(1, 2, 3, 8, 16)[i % 5])
     ok = rc == 0 and T._same_packets(d, o, l, out, lens) and np.array_equal(r, rng)
     return i, bool(ok)

@@ -1,11 +1,13 @@
 """CPU twin of tools/parity_sweep.py: the same random batches (draw_batch, wide mode), coded by the HOST SIMULATION of the kernel
 headers (tests/hostsim: 1-lane teams, the kernels' call / run schedule emulated) instead of the GPU, against the oracle.  A test
 tool like the host simulation itself: it localises logic errors of the shared headers without GPU time; it says nothing about
-warp-level races.
+warp-level races.  Random batches have no stored reference results (tests/oracle_lib.py): run standalone, the oracle is the host
+simulation itself, so the sweep checks the emulated call / run schedule against plain per-packet decoding, not the headers' logic.
 
 usage: python tools/hostsim_sweep.py [batches=20] [streams_per_batch=16] [seed=1] [workers=8]
 """
 import ctypes as C
+import functools
 import os
 import sys
 import time
@@ -32,12 +34,12 @@ def hostsim():
     return _hs
 
 
-def one_stream(job):
+def one_stream(job, pin=True):
     (b, i, ch, fs, F, cfg, cut, loss, Fs, dFs, dch, maxb, extra, capmul) = job
     hs = hostsim()
     br, (vbr, cvbr), cx, kind, sd = cfg
     pcm = O.test_signal(F * fs, ch, sd, kind)
-    rd, ro, rl, rr = PS.ref_encode(pcm, fs, br, ch, Fs, vbr, cvbr, cx, maxb, extra[0], extra[1])
+    rd, ro, rl, rr = PS.ref_encode(pcm, fs, br, ch, Fs, vbr, cvbr, cx, maxb, extra[0], extra[1], pin=pin)
     out = np.zeros((F, 1276), dtype=np.uint8)
     lens = np.zeros(F, dtype=np.int32)
     rng = np.zeros(F, dtype=np.uint32)
@@ -52,7 +54,7 @@ def one_stream(job):
     dfs = int(fs * dFs // Fs * capmul)
     if dfs * 25 > dFs * 3:
         dfs = fs * dFs // Fs
-    rp, rrg, rret = O.decode_stream(rd, ro, dl, dfs, dch, Fs=dFs)
+    rp, rrg, rret = O.decode_stream(rd, ro, dl, dfs, dch, Fs=dFs, pin=pin)
     hp = np.zeros((F * dfs, dch), dtype=np.int16)
     hr = np.zeros(F, dtype=np.uint32)
     hret = np.zeros(F, dtype=np.int32)
@@ -72,7 +74,6 @@ def main():
     SEED = int(sys.argv[3]) if len(sys.argv) > 3 else 1
     NW = int(sys.argv[4]) if len(sys.argv) > 4 else 8
     hostsim()
-    O.ref()
     rs = np.random.RandomState(SEED)
     jobs = []
     for b in range(NB):
@@ -82,7 +83,7 @@ def main():
     t0 = time.time()
     bad = 0
     with Pool(NW) as pool:
-        for k, (b, i, e_ok, d_ok, info) in enumerate(pool.imap_unordered(one_stream, jobs, chunksize=4)):
+        for k, (b, i, e_ok, d_ok, info) in enumerate(pool.imap_unordered(functools.partial(one_stream, pin=False), jobs, chunksize=4)):
             if not (e_ok and d_ok):
                 bad += 1
                 print("MISMATCH batch %d stream %d encode_ok=%s decode_ok=%s %s" % (b, i, e_ok, d_ok, info), flush=True)

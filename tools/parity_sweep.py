@@ -6,6 +6,8 @@ batch and a summary; exit code 1 on any mismatch.
 usage: python tools/parity_sweep.py [batches=24] [streams_per_batch=48] [seed=1] [wide]     (SWEEP_ONLY=51,123 runs just those batches)
 `wide` also draws the encoder's API rate (8-48 kHz), 40 / 60 ms frames (repacketized multi-frame packets), and a decoder whose
 rate and channel count differ from the stream's.
+Random batches have no stored reference results (tests/oracle_lib.py), so the oracle here is the host simulation of the same
+headers unchecked: the sweep finds disagreements between the CUDA and host builds, not errors both share.
 """
 import ctypes as C
 import os
@@ -62,17 +64,12 @@ def draw_batch(rs, NS, wide=False):
     return ch, fs, F, cfgs, cut, loss, Fs, dFs, dch, maxb, extra, capmul
 
 
-def ref_encode(pcm, fs, br, ch, Fs, vbr, cvbr, cx, maxb, force_channels, bandwidth):
+def ref_encode(pcm, fs, br, ch, Fs, vbr, cvbr, cx, maxb, force_channels, bandwidth, pin=True):
     """The oracle's encoder with the full settings struct -> (data [F*1276], offs, lens, ranges)."""
-    pcm = np.ascontiguousarray(pcm, dtype=np.int16)
-    F = pcm.shape[0] // fs
-    out = np.zeros(F * 1276, dtype=np.uint8)
-    lens = np.zeros(F, dtype=np.int32)
-    ranges = np.zeros(F, dtype=np.uint32)
-    cfg = O.RefEncCfg(O.OPUS_APPLICATION_RESTRICTED_LOWDELAY, br, vbr, cvbr, cx, maxb, force_channels, bandwidth)
-    rc = O.ref().ref_encode_stream(O.ptr(pcm), F, fs, ch, Fs, C.byref(cfg), O.ptr(out), 1276, O.ptr(lens), O.ptr(ranges))
-    assert rc == 0, rc
-    return out, np.arange(F, dtype=np.int64) * 1276, lens, ranges
+    out, offs, lens, ranges = O.encode_stream(pcm, fs, br, ch, Fs=Fs, vbr=vbr, cvbr=cvbr, complexity=cx, max_bytes=maxb,
+                                              force_channels=force_channels, bandwidth=bandwidth, pin=pin)
+    assert (lens >= 0).all(), lens.min()
+    return out, offs, lens, ranges
 
 
 def main():
@@ -111,7 +108,8 @@ def main():
         enc.close()
         d = np.concatenate([d1.reshape(NS, cut, maxb), d2.reshape(NS, F - cut, maxb)], axis=1)
         l = np.concatenate([l1.reshape(NS, cut), l2.reshape(NS, F - cut)], axis=1)
-        refs = [ref_encode(pcms[i], fs, cfgs[i][0], ch, Fs, cfgs[i][1][0], cfgs[i][1][1], cfgs[i][2], maxb, extra[i][0], extra[i][1]) for i in range(NS)]
+        refs = [ref_encode(pcms[i], fs, cfgs[i][0], ch, Fs, cfgs[i][1][0], cfgs[i][1][1], cfgs[i][2], maxb, extra[i][0], extra[i][1], pin=False)
+                for i in range(NS)]
         bad_e = []
         for i, (rd, ro, rl, rr) in enumerate(refs):
             rd = rd.reshape(F, 1276)
@@ -133,7 +131,7 @@ def main():
         rets = np.concatenate([r1.reshape(NS, cut), r2.reshape(NS, F - cut)], axis=1)
         bad_d = []
         for i in range(NS):
-            rp, rr, rret = O.decode_stream(blob, offs[i], lens[i], dfs, dch, Fs=dFs)
+            rp, rr, rret = O.decode_stream(blob, offs[i], lens[i], dfs, dch, Fs=dFs, pin=False)
             rp = rp.reshape(F, dfs * dch)
             # what a caller may read: the first ret samples of every row; the rest of a row is compared too (the library
             # zero-fills it, the reference leaves the caller's zero-initialised buffer alone)

@@ -34,7 +34,7 @@ for b in range(NB):
     seeds = [int(rs.randint(1 << 30)) for _ in range(NS)]
     pcms = [O.test_signal(F * fs, ch, sd, KINDS[sd % 4]) for sd in seeds]
     scripts = [O.ctl_script(sd, F, ch, K=2) for sd in seeds]
-    refs = [O.encode_stream_script(pcms[i], fs, ch, scripts[i]) for i in range(NS)]
+    refs = [O.encode_stream_script(pcms[i], fs, ch, scripts[i], pin=False) for i in range(NS)]
     enc = cb.EncoderBatch(NS, 48000, ch, bitrate=64000, vbr=1, cvbr=1, complexity=10)
     x = np.stack([p.reshape(F, fs * ch) for p in pcms])
     v = C.c_uint32(0)
