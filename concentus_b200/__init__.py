@@ -30,6 +30,7 @@ OPUS_GET_PITCH_REQUEST = 4033
 OPUS_SET_GAIN_REQUEST = 4034
 OPUS_GET_GAIN_REQUEST = 4045
 OPUS_GET_LAST_PACKET_DURATION_REQUEST = 4039
+OPUS_MULTISTREAM_GET_DECODER_STATE_REQUEST = 5122
 
 _lib = None
 
@@ -46,6 +47,9 @@ EXPORTS = [
     "opus_repacketizer_get_size", "opus_repacketizer_init", "opus_repacketizer_create", "opus_repacketizer_destroy", "opus_repacketizer_cat",
     "opus_repacketizer_get_nb_frames", "opus_repacketizer_out_range", "opus_repacketizer_out",
     "opus_b200_enc_set_pipeline", "opus_b200_enc_path_counts", "opus_b200_enc_band_stats",
+    "opus_multistream_decoder_get_size", "opus_multistream_decoder_create", "opus_multistream_decoder_init", "opus_multistream_decode",
+    "opus_multistream_decoder_ctl", "opus_multistream_decoder_destroy", "opus_multistream_decode_span",
+    "opus_multistream_decode_span_device", "opus_multistream_decoder_sync", "opus_b200_ms_stage_times",
 ]
 
 OPUS_APPLICATION_VOIP = 2048
@@ -102,6 +106,17 @@ def lib():
         L.opus_b200_enc_kernel_launches.restype = C.c_longlong
         L.opus_b200_enc_stream.restype = C.c_void_p
         L.opus_b200_enc_last_kernel_ms.restype = C.c_float
+        L.opus_multistream_decoder_create.restype = C.c_void_p
+        L.opus_multistream_decoder_create.argtypes = [C.c_int32, C.c_int, C.c_int, C.c_int, C.c_void_p, C.POINTER(C.c_int)]
+        L.opus_multistream_decoder_init.argtypes = [C.c_void_p, C.c_int32, C.c_int, C.c_int, C.c_int, C.c_void_p]
+        L.opus_multistream_decoder_get_size.argtypes = [C.c_int, C.c_int]
+        L.opus_multistream_decoder_destroy.argtypes = [C.c_void_p]
+        L.opus_multistream_decoder_destroy.restype = None
+        L.opus_multistream_decode.argtypes = L.opus_decode.argtypes
+        L.opus_multistream_decode_span.argtypes = L.opus_decode_span.argtypes
+        L.opus_multistream_decode_span_device.argtypes = L.opus_decode_span.argtypes
+        L.opus_multistream_decoder_sync.argtypes = [C.c_void_p, C.c_int]
+        L.opus_b200_ms_stage_times.argtypes = [C.c_void_p, C.c_void_p, C.c_int]
         _lib = L
     return _lib
 
@@ -149,6 +164,61 @@ class DecoderBatch:
         for i in range(self.n):
             if self.handles[i]:
                 L.opus_decoder_destroy(C.c_void_p(self.handles[i]))
+                self.handles[i] = None
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+
+class MSDecoderBatch:
+    """n multistream decoders (same Fs / channels / streams / coupled streams) driven through the multistream span C ABI.
+    mapping: one channel mapping for all decoders, or one per decoder."""
+
+    def __init__(self, n, Fs, channels, streams, coupled, mapping):
+        L = lib()
+        self.n, self.Fs, self.channels, self.streams, self.coupled = n, Fs, channels, streams, coupled
+        maps = np.asarray(mapping, dtype=np.uint8).reshape(-1, channels)
+        if maps.shape[0] == 1:
+            maps = np.repeat(maps, n, axis=0)
+        assert maps.shape[0] == n
+        self.mappings = np.ascontiguousarray(maps)
+        err = C.c_int(0)
+        self.handles = (C.c_void_p * n)()
+        for i in range(n):
+            h = L.opus_multistream_decoder_create(Fs, channels, streams, coupled, _p(self.mappings[i]), C.byref(err))
+            if not h:
+                raise RuntimeError("opus_multistream_decoder_create failed: %d" % err.value)
+            self.handles[i] = h
+
+    def decode_span(self, data, offs, lens, F, frame_size):
+        """Host buffers in, host buffers out: returns (pcm [n*F*frame_size, channels], rets [n*F])."""
+        L = lib()
+        pcm = np.zeros((self.n * F * frame_size, self.channels), dtype=np.int16)
+        rets = np.zeros(self.n * F, dtype=np.int32)
+        rc = L.opus_multistream_decode_span(self.handles, self.n, F, _p(data), _p(np.ascontiguousarray(offs, dtype=np.int64)),
+                                            _p(np.ascontiguousarray(lens, dtype=np.int32)), _p(pcm), frame_size, _p(rets))
+        if rc != OPUS_OK:
+            raise RuntimeError("opus_multistream_decode_span: %s" % L.opus_strerror(rc).decode())
+        return pcm, rets
+
+    def final_ranges(self):
+        """OPUS_GET_FINAL_RANGE of each multistream decoder: the XOR of its streams' final ranges."""
+        L = lib()
+        out = np.zeros(self.n, dtype=np.uint32)
+        v = C.c_uint32(0)
+        for i in range(self.n):
+            L.opus_multistream_decoder_ctl(C.c_void_p(self.handles[i]), OPUS_GET_FINAL_RANGE_REQUEST, C.byref(v))
+            out[i] = v.value
+        return out
+
+    def close(self):
+        L = lib()
+        for i in range(self.n):
+            if self.handles[i]:
+                L.opus_multistream_decoder_destroy(C.c_void_p(self.handles[i]))
                 self.handles[i] = None
 
     def __del__(self):

@@ -20,6 +20,7 @@
 #include "../../include/opus_b200.h"
 #include "host_runtime.h"
 #include "opus_decoder_dev.cuh"
+#include "opus_multistream.h"
 
 using namespace cb;
 
@@ -94,21 +95,21 @@ __global__ void call_ctx_kernel(const CbDecState *pool, const int *slots, CbCall
 }
 
 // Stage B — synthesis, one warp per stream, packets f0..f1 in order.  PCM row of packet (s,f) starts at
-// pcm[(s*pcm_F + (f-pcm_f0)) * cap * channels].
+// pcm[(s*pcm_F + (f-pcm_f0)) * row]: row = cap * channels for a call of uniform channel count, cap * 2 when mono and stereo
+// streams share one staging layout (multistream calls).
 __global__ void __launch_bounds__(CB_WPB * 32, CB_SYNTH_MINBLOCKS)
 synth_kernel(CbDecState *pool, const int *slots, IrView ir, int16_t *pcm, int n, int F, int f0, int f1, int pcm_F, int pcm_f0,
-             int cap, int *rets, PlcScratch *plc) {
+             int cap, int row, int *rets, PlcScratch *plc) {
     extern __shared__ __align__(16) unsigned char smem[];
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int s = blockIdx.x * CB_WPB + warp;
     if (s >= n) return;
     SynthScratch &S = *(reinterpret_cast<SynthScratch *>(smem) + warp);
     CbDecState *st = pool + slots[s];
-    const int channels = st->channels;
     WarpTeam tm{lane};
     for (int f = f0; f < f1; f++) {
         const size_t slot = (size_t)s * ir.Fc + (f - f0);
-        int16_t *out = pcm + ((size_t)s * pcm_F + (f - pcm_f0)) * cap * channels;
+        int16_t *out = pcm + ((size_t)s * pcm_F + f - pcm_f0) * row;
         int r = opus_synth_packet(tm, st, S, plc[s], ir.pk[slot], ir.fr + slot * ir.kmax, ir.X + slot * ir.xstride, out, cap,
                                   ir.sig + slot * ir.sigstride, ir.range + slot);
         if (lane == 0) rets[(size_t)s * F + f] = r;
@@ -152,7 +153,7 @@ __device__ __forceinline__ int deemph_pair_stereo(const int *x, int n, int16_t *
 }
 
 __global__ void __launch_bounds__(128)
-deemph_kernel(CbDecState *pool, const int *slots, IrView ir, int16_t *pcm, int n, int f0, int f1, int pcm_F, int pcm_f0, int cap) {
+deemph_kernel(CbDecState *pool, const int *slots, IrView ir, int16_t *pcm, int n, int f0, int f1, int pcm_F, int pcm_f0, int cap, int row) {
     const int t = blockIdx.x * blockDim.x + threadIdx.x;
     const int s = t >> 1, c = t & 1;
     if (s >= n) return;
@@ -166,7 +167,7 @@ deemph_kernel(CbDecState *pool, const int *slots, IrView ir, int16_t *pcm, int n
     int m = st->preemph_memD[c];
     for (int f = f0; f < f1; f++) {
         const size_t slot = (size_t)s * ir.Fc + (f - f0);
-        int16_t *out = pcm + ((size_t)s * pcm_F + (f - pcm_f0)) * cap * channels;
+        int16_t *out = pcm + ((size_t)s * pcm_F + (f - pcm_f0)) * row;
         const CbSigRange rg = ir.range[slot];
         if (rg.end <= rg.begin) continue;
         const int *x = ir.sig + slot * ir.sigstride + c * (cap * ds) + rg.begin;
@@ -182,6 +183,74 @@ deemph_kernel(CbDecState *pool, const int *slots, IrView ir, int16_t *pcm, int n
             m = deemphasis_channel(x, cnt, y0 + c, channels, ds, m, gain);
     }
     st->preemph_memD[c] = m;
+}
+
+// ---- multistream (DESIGN.md §3): a call over n multistream decoders of S streams is one pipeline call over the n*S embedded
+// decoders, elementary decoder e = m*S + s.  ms_split_kernel turns the multistream packets into elementary ones before it,
+// ms_gather_kernel turns each chunk's elementary PCM into multistream rows after it.
+
+// End of the furthest packet of a device-resident span (the size of the split's scratch copy of the input).
+__global__ void ms_extent_kernel(const int64_t *offs, const int32_t *lens, int N, unsigned long long *extent) {
+    const int t = blockIdx.x * blockDim.x + threadIdx.x;
+    if (t < N && lens[t] > 0) atomicMax(extent, (unsigned long long)(offs[t] + lens[t]));
+}
+
+// One thread per multistream packet (m,f): validation and undelimiting (ms_split_packet) into `blob`, a copy of `data` followed by
+// the reject marker at `reject_off`; fills the elementary offsets / lengths [(m*S+s)*F + f] and the packet's own error code (0 = none).
+__global__ void ms_split_kernel(const uint8_t *data, const int64_t *offs, const int32_t *lens, int n, int F, int S, int Fs, int frame_size,
+                                uint8_t *blob, int64_t reject_off, int64_t *eoffs, int32_t *elens, int *ms_err) {
+    const int t = blockIdx.x * blockDim.x + threadIdx.x;
+    if (t == 0) ms_write_reject_marker(blob + reject_off);   // read only by the stages after this kernel
+    if (t >= n * F) return;
+    const int m = t / F, f = t - m * F;
+    const int len = lens[t];
+    const int64_t off = len > 0 ? offs[t] : 0;
+    const size_t e0 = (size_t)m * S * F + f;
+    const int r = ms_split_packet(data + off, len, S, Fs, frame_size, blob + off, off, eoffs + e0, elens + e0, (size_t)F, reject_off);
+    ms_err[t] = r < 0 ? r : 0;
+}
+
+// One block per multistream packet of the chunk [f0, f1): output channel c of sample i is stream channel mapping[c] of the
+// elementary rows (coupled stream s: channels 2s / 2s+1, interleaved in a stereo row; mono stream s: channel coupled + s), a
+// channel mapped to 255 and the row tail past the packet's samples are zero.  ret = the packet's split error, else the first
+// elementary error in stream order, else the sample count; a packet with an error gets an all-zero row.
+// epcm: elementary row (e, f) at ((e * e_F) + f - f0) * erow; out: row (m, f) at ((m * out_F) + f - out_f0) * frame_size * channels.
+__global__ void __launch_bounds__(256)
+ms_gather_kernel(const int16_t *epcm, int e_F, int erow, const int *erets, const int *ms_err, const uint8_t *mapping, int16_t *out,
+                 int out_F, int out_f0, int F, int f0, int f1, int S, int coupled, int channels, int frame_size, int *ret) {
+    __shared__ int s_ret;
+    __shared__ uint8_t s_map[256];
+    const int nf = f1 - f0;
+    const int m = blockIdx.x / nf, f = f0 + (blockIdx.x - m * nf);
+    for (int c = threadIdx.x; c < channels; c += blockDim.x) s_map[c] = mapping[(size_t)m * channels + c];
+    if (threadIdx.x == 0) {
+        int r = ms_err[(size_t)m * F + f];
+        if (r == 0) {
+            r = erets[((size_t)m * S) * F + f];
+            for (int s = 1; s < S && r >= 0; s++) {
+                const int e = erets[((size_t)m * S + s) * F + f];
+                if (e < 0) r = e;
+            }
+        }
+        s_ret = r;
+        ret[(size_t)m * F + f] = r;
+    }
+    __syncthreads();
+    const int r = s_ret > 0 ? s_ret : 0;
+    const int16_t *ebase = epcm + ((size_t)m * S * e_F + (f - f0)) * erow;
+    const size_t estride = (size_t)e_F * erow;   // from stream s to s+1 of the same multistream decoder
+    int16_t *o = out + ((size_t)m * out_F + (f - out_f0)) * frame_size * channels;
+    for (int i = threadIdx.x; i < frame_size; i += blockDim.x) {
+        for (int c = 0; c < channels; c++) {
+            const int k = s_map[c];
+            int16_t v = 0;
+            if (i < r && k != 255) {
+                if (k < 2 * coupled) v = ebase[(size_t)(k >> 1) * estride + 2 * i + (k & 1)];
+                else v = ebase[(size_t)(k - coupled) * estride + i];
+            }
+            o[(size_t)i * channels + c] = v;
+        }
+    }
 }
 
 // state staging <-> pool
@@ -224,6 +293,10 @@ struct Ctx {
     std::vector<int> free_slots;
     DevBuf d_slots, d_data, d_offs, d_lens, d_pcm[2], d_rets, d_stage;
     DevBuf d_irpk[2], d_irfr[2], d_irx[2], d_sig[2], d_range[2], d_plc, d_callctx;
+    // multistream calls: the split's copy of the input, elementary offsets / lengths / returns, per-packet split errors, channel
+    // mappings, elementary PCM of a chunk (double-buffered), the input extent of a device-resident span
+    DevBuf d_blob, d_eoffs, d_elens, d_erets, d_mserr, d_map, d_epcm[2], d_extent;
+    cudaEvent_t ev_gather[2] = {nullptr, nullptr};
     size_t ir_budget = (size_t)16 << 30;  // bytes of IR + staging per chunk buffer (env CB200_IR_MB)
     // Host-buffer calls copy each chunk's PCM out while the next chunk decodes; the last chunk's copy overlaps nothing, so
     // they run on smaller chunks (measured: e2e 108 K -> 126 K x realtime; the device-resident path keeps the large ones)
@@ -238,8 +311,8 @@ struct Ctx {
     struct Timed { cudaEvent_t a, b; int stage; };
     std::vector<Timed> timed;
     std::vector<cudaEvent_t> ev_pool;
-    double stage_ms[3] = {0, 0, 0};
-    long long stage_launches[3] = {0, 0, 0};
+    double stage_ms[5] = {0, 0, 0, 0, 0};   // parse, synth, de-emphasis, multistream split, multistream gather
+    long long stage_launches[5] = {0, 0, 0, 0, 0};
     int smem_per_block = 0;
     // slots of this device's pool whose owners moved to another device: released by the next call here (see release_elsewhere)
     std::mutex deferred_mu;
@@ -301,6 +374,7 @@ bool ctx_init_locked() {
         cudaEventCreateWithFlags(&g.ev_parse[i], cudaEventDisableTiming);
         cudaEventCreateWithFlags(&g.ev_synth[i], cudaEventDisableTiming);
         cudaEventCreateWithFlags(&g.ev_deemph[i], cudaEventDisableTiming);
+        cudaEventCreateWithFlags(&g.ev_gather[i], cudaEventDisableTiming);
     }
     cudaEventCreateWithFlags(&g.ev_call, cudaEventDisableTiming);
     if (const char *e = getenv("CB200_IR_MB")) g.ir_budget = (size_t)atol(e) << 20;
@@ -576,9 +650,10 @@ IrView ir_view(const Plan &pl, int b) {
 }
 
 // Enqueue stage A for chunk c on the parse stream and stage B on the main stream.  PCM goes to pcm_dst laid out with
-// pcm_F packets per stream starting at packet pcm_f0 (the caller decides: whole-call buffer or a chunk buffer).
+// pcm_F packets per stream starting at packet pcm_f0, `row` int16 per packet (the caller decides: whole-call buffer or a chunk
+// buffer).
 void enqueue_chunk(const Plan &pl, int c, const int *d_slots, const uint8_t *d_data, const int64_t *d_offs, const int32_t *d_lens,
-                   int16_t *pcm_dst, int pcm_F, int pcm_f0, int *d_rets, cudaEvent_t pcm_free = nullptr) {
+                   int16_t *pcm_dst, int pcm_F, int pcm_f0, int row, int *d_rets, cudaEvent_t pcm_free = nullptr) {
     const int b = c & 1;
     const int f0 = c * pl.Fc, f1 = (f0 + pl.Fc < pl.F) ? f0 + pl.Fc : pl.F;
     const int runs = (f1 - f0 + pl.R - 1) / pl.R;
@@ -601,13 +676,13 @@ void enqueue_chunk(const Plan &pl, int c, const int *d_slots, const uint8_t *d_d
     if (pcm_free) cudaStreamWaitEvent(g.synth_stream, pcm_free, 0);   // stage B writes PCM too (leading zero frames)
     timing_begin(1, g.synth_stream);
     synth_kernel<<<(pl.n + CB_WPB - 1) / CB_WPB, CB_WPB * 32, g.smem_per_block, g.synth_stream>>>(g.pool, d_slots, v, pcm_dst, pl.n, pl.F, f0,
-                                                                                                  f1, pcm_F, pcm_f0, pl.cap, d_rets, (PlcScratch *)g.d_plc.p);
+                                                                                                  f1, pcm_F, pcm_f0, pl.cap, row, d_rets, (PlcScratch *)g.d_plc.p);
     timing_end(g.synth_stream);
     cudaEventRecord(g.ev_synth[b], g.synth_stream);
     // stage C(c) on the main stream (the one the caller synchronises / times)
     cudaStreamWaitEvent(g.stream, g.ev_synth[b], 0);
     timing_begin(2, g.stream);
-    deemph_kernel<<<(2 * pl.n + 127) / 128, 128, 0, g.stream>>>(g.pool, d_slots, v, pcm_dst, pl.n, f0, f1, pcm_F, pcm_f0, pl.cap);
+    deemph_kernel<<<(2 * pl.n + 127) / 128, 128, 0, g.stream>>>(g.pool, d_slots, v, pcm_dst, pl.n, f0, f1, pcm_F, pcm_f0, pl.cap, row);
     timing_end(g.stream);
     cudaEventRecord(g.ev_deemph[b], g.stream);
     g.launches += 3;
@@ -660,6 +735,16 @@ int opus_b200_stage_times(double ms[3], long long launches[3], int reset) {
         if (ms) ms[i] = g.stage_ms[i];
         if (launches) launches[i] = g.stage_launches[i];
         if (reset) { g.stage_ms[i] = 0; g.stage_launches[i] = 0; }
+    }
+    return OPUS_OK;
+}
+// The same for the two multistream stages (0 = split, 1 = gather).
+int opus_b200_ms_stage_times(double ms[2], long long launches[2], int reset) {
+    std::lock_guard<std::mutex> lk(g.mu);
+    for (int i = 0; i < 2; i++) {
+        if (ms) ms[i] = g.stage_ms[3 + i];
+        if (launches) launches[i] = g.stage_launches[3 + i];
+        if (reset) { g.stage_ms[3 + i] = 0; g.stage_launches[3 + i] = 0; }
     }
     return OPUS_OK;
 }
@@ -850,7 +935,7 @@ int opus_decode_span_device(OpusDecoder **st, int n, int F, const unsigned char 
     g.launches++;
     cudaEventRecord(g.ev_call, g.stream);
     for (int c = 0; c < pl.nchunks; c++)
-        enqueue_chunk(pl, c, (const int *)g.d_slots.p, d_data, d_offs, d_len, d_pcm, F, 0, d_ret);
+        enqueue_chunk(pl, c, (const int *)g.d_slots.p, d_data, d_offs, d_len, d_pcm, F, 0, frame_size * st[0]->st.channels, d_ret);
     cudaEventRecord(g.ev1, g.stream);
     mark_device_newer_locked(st, n);
     if (cudaGetLastError() != cudaSuccess) return OPUS_INTERNAL_ERROR;
@@ -898,7 +983,8 @@ static int decode_span_host_locked(OpusDecoder **st, int n, int F, const unsigne
         const int f0 = c * Fc, f1 = (f0 + Fc < F) ? f0 + Fc : F;
         if (c >= 2) cudaStreamWaitEvent(g.stream, g.ev_copy[b], 0);   // PCM buffer b drained?
         enqueue_chunk(pl, c, (const int *)g.d_slots.p, (const uint8_t *)g.d_data.p, (const int64_t *)g.d_offs.p,
-                      (const int32_t *)g.d_lens.p, (int16_t *)g.d_pcm[b].p, Fc, f0, (int *)g.d_rets.p, c >= 2 ? g.ev_copy[b] : nullptr);
+                      (const int32_t *)g.d_lens.p, (int16_t *)g.d_pcm[b].p, Fc, f0, frame_size * channels, (int *)g.d_rets.p,
+                      c >= 2 ? g.ev_copy[b] : nullptr);
         cudaEventRecord(g.ev_chunk[b], g.stream);
         cudaStreamWaitEvent(g.copy_stream, g.ev_chunk[b], 0);
         // rows of (f1-f0) packets per stream: device pitch Fc*row, host pitch F*row
@@ -1031,6 +1117,305 @@ int opus_decode(OpusDecoder *st, const unsigned char *data, opus_int32 len, opus
     int rc = decode_span_host_locked(&one, 1, 1, data, l, &off, &l, out.data(), cap, decode_fec, &r, false);
     if (rc != OPUS_OK) return rc;
     if (r > 0) memcpy(pcm, out.data(), (size_t)r * channels * sizeof(int16_t));
+    return r;
+}
+
+}  // extern "C"
+
+// ------------------------------------------------------------------------------------------------
+// Multistream decoder (libopus opus_multistream.h; layout and packet format RFC 7845 §5.1.1, RFC 6716 Appendix B).  The block
+// is a header followed by `streams` ordinary OpusDecoder blocks (coupled streams first, stereo; then mono), so residency,
+// write-back, memcpy and the duplicate check of the embedded decoders are exactly those of single-stream decoders.
+// ------------------------------------------------------------------------------------------------
+struct OpusMSDecoder {
+    uint32_t magic;
+    int32_t Fs, channels, streams, coupled;
+    uint8_t mapping[255];   // output channel c = stream channel mapping[c]; 255 = silence
+};
+static const uint32_t kMsDecMagic = 0x0B2005DCu;
+static const size_t kMsHeader = (sizeof(OpusMSDecoder) + 63) & ~(size_t)63;
+
+static inline OpusDecoder *ms_stream(OpusMSDecoder *st, int s) {
+    return reinterpret_cast<OpusDecoder *>(reinterpret_cast<char *>(st) + kMsHeader + (size_t)s * sizeof(OpusDecoder));
+}
+
+// Multistream span over host or device buffers (device_io).  n decoders sharing (Fs, channels, streams, coupled); packet (m,f) at
+// data[offs[m*F+f] ..][0 .. len[m*F+f]), its PCM at pcm + (m*F+f)*frame_size*channels, ret[m*F+f] = what the scalar call returns.
+// data_bytes: extent of the host input (ignored for device_io, where it is measured on the device).
+static int ms_decode_span_locked(OpusMSDecoder **st, int n, int F, const unsigned char *data, int64_t data_bytes, const int64_t *offs,
+                                 const opus_int32 *len, opus_int16 *pcm, int frame_size, int decode_fec, int *ret, bool device_io,
+                                 bool keep_resident) {
+    if (!ctx_init_locked()) return OPUS_INTERNAL_ERROR;
+    for (int i = 0; i < n; i++) {
+        if (!st[i] || st[i]->magic != kMsDecMagic) return OPUS_BAD_ARG;
+        // one IR geometry and one elementary layout per call
+        if (st[i]->Fs != st[0]->Fs || st[i]->channels != st[0]->channels || st[i]->streams != st[0]->streams ||
+            st[i]->coupled != st[0]->coupled)
+            return OPUS_BAD_ARG;
+    }
+    const int Fs = st[0]->Fs, channels = st[0]->channels, S = st[0]->streams, coupled = st[0]->coupled;
+    const int E = n * S;
+    const size_t NF = (size_t)n * F, EF = (size_t)E * F;
+    std::vector<OpusDecoder *> el((size_t)E);
+    for (int m = 0; m < n; m++)
+        for (int s = 0; s < S; s++) el[(size_t)m * S + s] = ms_stream(st[m], s);
+    if (!g.h_slots.reserve(sizeof(int) * (size_t)E)) return OPUS_ALLOC_FAIL;
+    int *hsl = (int *)g.h_slots.p;
+    int rc = make_resident_locked(el.data(), E, hsl);
+    if (rc != OPUS_OK) return rc;
+    // opus_multistream_decode clamps the room per channel to 120 ms: what a lost packet conceals; rows keep frame_size
+    const int cap = frame_size < Fs / 25 * 3 ? frame_size : Fs / 25 * 3;
+    if (!g.d_slots.reserve(sizeof(int) * (size_t)E) || !g.d_eoffs.reserve(sizeof(int64_t) * EF) || !g.d_elens.reserve(sizeof(int32_t) * EF) ||
+        !g.d_erets.reserve(sizeof(int) * EF) || !g.d_mserr.reserve(sizeof(int) * NF) || !g.d_map.reserve((size_t)n * channels) ||
+        !g.d_extent.reserve(sizeof(unsigned long long)) || !g.h_misc.reserve(sizeof(unsigned long long)))
+        return OPUS_ALLOC_FAIL;
+    const uint8_t *d_in;
+    const int64_t *d_offs;
+    const int32_t *d_lens;
+    if (device_io) {
+        d_in = data; d_offs = offs; d_lens = len;
+        cudaMemsetAsync(g.d_extent.p, 0, sizeof(unsigned long long), g.stream);
+        ms_extent_kernel<<<(unsigned)((NF + 255) / 256), 256, 0, g.stream>>>(offs, len, (int)NF, (unsigned long long *)g.d_extent.p);
+        g.launches++;
+        cudaMemcpyAsync(g.h_misc.p, g.d_extent.p, sizeof(unsigned long long), cudaMemcpyDeviceToHost, g.stream);
+        if (cudaStreamSynchronize(g.stream) != cudaSuccess) return OPUS_INTERNAL_ERROR;
+        data_bytes = (int64_t)*(unsigned long long *)g.h_misc.p;
+    } else {
+        if (!g.d_data.reserve((size_t)data_bytes + 16) || !g.d_offs.reserve(sizeof(int64_t) * NF) || !g.d_lens.reserve(sizeof(int32_t) * NF) ||
+            !g.d_rets.reserve(sizeof(int) * NF))
+            return OPUS_ALLOC_FAIL;
+        if (data_bytes > 0) cudaMemcpyAsync(g.d_data.p, data, (size_t)data_bytes, cudaMemcpyHostToDevice, g.stream);
+        cudaMemcpyAsync(g.d_offs.p, offs, sizeof(int64_t) * NF, cudaMemcpyHostToDevice, g.stream);
+        cudaMemcpyAsync(g.d_lens.p, len, sizeof(int32_t) * NF, cudaMemcpyHostToDevice, g.stream);
+        d_in = (const uint8_t *)g.d_data.p; d_offs = (const int64_t *)g.d_offs.p; d_lens = (const int32_t *)g.d_lens.p;
+    }
+    if (!g.d_blob.reserve((size_t)data_bytes + 16)) return OPUS_ALLOC_FAIL;   // the input, then the reject marker at data_bytes
+    Plan pl;
+    if (!plan_call(pl, E, F, cap, decode_fec, Fs, !device_io)) return OPUS_ALLOC_FAIL;
+    const int Fc = pl.Fc, nchunks = pl.nchunks, erow = cap * 2;   // elementary rows sized for stereo: mono and stereo share them
+    const size_t orow = (size_t)frame_size * channels * sizeof(int16_t);
+    for (int b = 0; b < (nchunks > 1 ? 2 : 1); b++) {
+        if (!g.d_epcm[b].reserve((size_t)E * Fc * erow * sizeof(int16_t))) return OPUS_ALLOC_FAIL;
+        if (!device_io && !g.d_pcm[b].reserve((size_t)n * Fc * orow)) return OPUS_ALLOC_FAIL;
+    }
+    {
+        std::vector<uint8_t> maps((size_t)n * channels);
+        for (int m = 0; m < n; m++) memcpy(maps.data() + (size_t)m * channels, st[m]->mapping, (size_t)channels);
+        cudaMemcpyAsync(g.d_map.p, maps.data(), maps.size(), cudaMemcpyHostToDevice, g.stream);
+        cudaMemcpyAsync(g.d_slots.p, hsl, sizeof(int) * (size_t)E, cudaMemcpyHostToDevice, g.stream);
+        cudaStreamSynchronize(g.stream);   // `maps` is pageable and goes out of scope
+    }
+    cudaEventRecord(g.ev0, g.stream);
+    if (data_bytes > 0) cudaMemcpyAsync(g.d_blob.p, d_in, (size_t)data_bytes, cudaMemcpyDeviceToDevice, g.stream);
+    timing_begin(3, g.stream);
+    ms_split_kernel<<<(unsigned)((NF + 127) / 128), 128, 0, g.stream>>>(d_in, d_offs, d_lens, n, F, S, Fs, frame_size, (uint8_t *)g.d_blob.p,
+                                                                      data_bytes, (int64_t *)g.d_eoffs.p, (int32_t *)g.d_elens.p, (int *)g.d_mserr.p);
+    timing_end(g.stream);
+    call_ctx_kernel<<<(E + 127) / 128, 128, 0, g.stream>>>(g.pool, (const int *)g.d_slots.p, (CbCallCtx *)g.d_callctx.p, E);
+    g.launches += 2;
+    cudaEventRecord(g.ev_call, g.stream);
+    int *d_ret = device_io ? ret : (int *)g.d_rets.p;
+    for (int c = 0; c < nchunks; c++) {
+        const int b = c & 1;
+        const int f0 = c * Fc, f1 = (f0 + Fc < F) ? f0 + Fc : F;
+        if (!device_io && c >= 2) cudaStreamWaitEvent(g.stream, g.ev_copy[b], 0);   // output staging b drained?
+        // elementary staging b is free once the gather of chunk c-2 has read it
+        enqueue_chunk(pl, c, (const int *)g.d_slots.p, (const uint8_t *)g.d_blob.p, (const int64_t *)g.d_eoffs.p, (const int32_t *)g.d_elens.p,
+                      (int16_t *)g.d_epcm[b].p, Fc, f0, erow, (int *)g.d_erets.p, c >= 2 ? g.ev_gather[b] : nullptr);
+        int16_t *out = device_io ? (int16_t *)pcm : (int16_t *)g.d_pcm[b].p;
+        timing_begin(4, g.stream);
+        ms_gather_kernel<<<(unsigned)(n * (f1 - f0)), 256, 0, g.stream>>>((const int16_t *)g.d_epcm[b].p, Fc, erow, (const int *)g.d_erets.p,
+                                                                          (const int *)g.d_mserr.p, (const uint8_t *)g.d_map.p, out,
+                                                                          device_io ? F : Fc, device_io ? 0 : f0, F, f0, f1, S, coupled,
+                                                                          channels, frame_size, d_ret);
+        timing_end(g.stream);
+        g.launches++;
+        cudaEventRecord(g.ev_gather[b], g.stream);
+        if (!device_io) {
+            cudaEventRecord(g.ev_chunk[b], g.stream);
+            cudaStreamWaitEvent(g.copy_stream, g.ev_chunk[b], 0);
+            cudaMemcpy2DAsync((char *)pcm + (size_t)f0 * orow, (size_t)F * orow, g.d_pcm[b].p, (size_t)Fc * orow, (size_t)(f1 - f0) * orow,
+                              (size_t)n, cudaMemcpyDeviceToHost, g.copy_stream);
+            cudaEventRecord(g.ev_copy[b], g.copy_stream);
+        }
+    }
+    cudaEventRecord(g.ev1, g.stream);
+    mark_device_newer_locked(el.data(), E);
+    if (device_io) return cudaGetLastError() == cudaSuccess ? OPUS_OK : OPUS_INTERNAL_ERROR;
+    cudaMemcpyAsync(ret, g.d_rets.p, sizeof(int) * NF, cudaMemcpyDeviceToHost, g.stream);
+    if (cudaStreamSynchronize(g.stream) != cudaSuccess || cudaStreamSynchronize(g.copy_stream) != cudaSuccess ||
+        cudaStreamSynchronize(g.parse_stream) != cudaSuccess || cudaStreamSynchronize(g.synth_stream) != cudaSuccess) {
+        fprintf(stderr, "concentus_b200: CUDA failure in multistream decode: %s\n", cudaGetErrorString(cudaGetLastError()));
+        return OPUS_INTERNAL_ERROR;
+    }
+    cudaEventElapsedTime(&g.last_ms, g.ev0, g.ev1);
+    timing_fold();
+    if (!keep_resident) return sync_states_locked(el.data(), E, true);
+    return OPUS_OK;
+}
+
+extern "C" {
+
+int opus_multistream_decoder_get_size(int streams, int coupled_streams) {
+    if (streams < 1 || coupled_streams > streams || coupled_streams < 0) return 0;
+    return (int)(kMsHeader + (size_t)streams * sizeof(OpusDecoder));
+}
+
+int opus_multistream_decoder_init(OpusMSDecoder *st, opus_int32 Fs, int channels, int streams, int coupled_streams,
+                                  const unsigned char *mapping) {
+    if (channels > 255 || channels < 1 || coupled_streams > streams || streams < 1 || coupled_streams < 0 || streams > 255 - coupled_streams)
+        return OPUS_BAD_ARG;
+    if (!mapping) return OPUS_BAD_ARG;
+    for (int c = 0; c < channels; c++)
+        if (mapping[c] >= streams + coupled_streams && mapping[c] != 255) return OPUS_BAD_ARG;
+    // re-initialising a live block in place: the embedded decoders give their pool slots back (opus_decoder_init)
+    const bool live = st->magic == kMsDecMagic;
+    const int old_streams = live ? st->streams : 0;
+    for (int s = 0; s < streams; s++) {
+        OpusDecoder *d = ms_stream(st, s);
+        if (!(live && s < old_streams)) d->magic = 0;   // not a live decoder: nothing to release
+        const int ret = opus_decoder_init(d, Fs, s < coupled_streams ? 2 : 1);
+        if (ret != OPUS_OK) return ret;
+    }
+    st->magic = kMsDecMagic;
+    st->Fs = Fs;
+    st->channels = channels;
+    st->streams = streams;
+    st->coupled = coupled_streams;
+    memset(st->mapping, 255, sizeof(st->mapping));
+    memcpy(st->mapping, mapping, (size_t)channels);
+    return OPUS_OK;
+}
+
+OpusMSDecoder *opus_multistream_decoder_create(opus_int32 Fs, int channels, int streams, int coupled_streams, const unsigned char *mapping,
+                                               int *error) {
+    if (channels > 255 || channels < 1 || coupled_streams > streams || streams < 1 || coupled_streams < 0 || streams > 255 - coupled_streams) {
+        if (error) *error = OPUS_BAD_ARG;
+        return nullptr;
+    }
+    OpusMSDecoder *st = (OpusMSDecoder *)malloc((size_t)opus_multistream_decoder_get_size(streams, coupled_streams));
+    if (!st) {
+        if (error) *error = OPUS_ALLOC_FAIL;
+        return nullptr;
+    }
+    st->magic = 0;
+    const int ret = opus_multistream_decoder_init(st, Fs, channels, streams, coupled_streams, mapping);
+    if (error) *error = ret;
+    if (ret != OPUS_OK) {
+        opus_multistream_decoder_destroy(st);
+        st = nullptr;
+    }
+    return st;
+}
+
+void opus_multistream_decoder_destroy(OpusMSDecoder *st) {
+    if (!st) return;
+    if (st->magic == kMsDecMagic) {
+        std::lock_guard<std::mutex> lk(g.mu);
+        if (g.ok)
+            for (int s = 0; s < st->streams; s++) {
+                OpusDecoder *d = ms_stream(st, s);
+                if (d->magic == kDecMagic) release_slot_locked(d);
+            }
+    }
+    free(st);
+}
+
+int opus_multistream_decoder_ctl(OpusMSDecoder *st, int request, ...) {
+    if (!st || st->magic != kMsDecMagic) return OPUS_BAD_ARG;
+    int ret = OPUS_OK;
+    va_list ap;
+    va_start(ap, request);
+    switch (request) {
+    case OPUS_GET_BANDWIDTH_REQUEST:
+    case OPUS_GET_SAMPLE_RATE_REQUEST:
+    case OPUS_GET_GAIN_REQUEST:
+    case OPUS_GET_LAST_PACKET_DURATION_REQUEST: {   // answered by the first stream
+        void *v = va_arg(ap, void *);
+        ret = opus_decoder_ctl(ms_stream(st, 0), request, v);
+    } break;
+    case OPUS_GET_FINAL_RANGE_REQUEST: {   // XOR of every stream's final range
+        opus_uint32 *v = va_arg(ap, opus_uint32 *);
+        if (!v) { ret = OPUS_BAD_ARG; break; }
+        opus_uint32 acc = 0, r = 0;
+        for (int s = 0; s < st->streams && ret == OPUS_OK; s++) {
+            ret = opus_decoder_ctl(ms_stream(st, s), OPUS_GET_FINAL_RANGE_REQUEST, &r);
+            acc ^= r;
+        }
+        if (ret == OPUS_OK) *v = acc;
+    } break;
+    case OPUS_RESET_STATE:
+        for (int s = 0; s < st->streams && ret == OPUS_OK; s++) ret = opus_decoder_ctl(ms_stream(st, s), OPUS_RESET_STATE);
+        break;
+    case OPUS_SET_GAIN_REQUEST: {
+        const opus_int32 v = va_arg(ap, opus_int32);
+        for (int s = 0; s < st->streams && ret == OPUS_OK; s++) ret = opus_decoder_ctl(ms_stream(st, s), OPUS_SET_GAIN_REQUEST, v);
+    } break;
+    case OPUS_MULTISTREAM_GET_DECODER_STATE_REQUEST: {
+        const opus_int32 id = va_arg(ap, opus_int32);
+        OpusDecoder **v = va_arg(ap, OpusDecoder **);
+        if (id < 0 || id >= st->streams) { ret = OPUS_BAD_ARG; break; }
+        *v = ms_stream(st, id);
+    } break;
+    default:
+        ret = OPUS_UNIMPLEMENTED;
+        break;
+    }
+    va_end(ap);
+    return ret;
+}
+
+int opus_multistream_decode_span(OpusMSDecoder **st, int n, int F, const unsigned char *data, const int64_t *offs, const opus_int32 *len,
+                                 opus_int16 *pcm, int frame_size, int *ret) {
+    if (!st || n <= 0 || F <= 0 || frame_size <= 0 || !offs || !len || !pcm || !ret) return OPUS_BAD_ARG;
+    int64_t bytes = 0;
+    const size_t NF = (size_t)n * F;
+    for (size_t i = 0; i < NF; i++) {
+        if (len[i] > 0 && offs[i] < 0) return OPUS_BAD_ARG;
+        const int64_t e = offs[i] + len[i];
+        if (len[i] > 0 && e > bytes) bytes = e;
+    }
+    std::lock_guard<std::mutex> lk(g.mu);
+    return ms_decode_span_locked(st, n, F, data, bytes, offs, len, pcm, frame_size, 0, ret, false, true);
+}
+
+int opus_multistream_decode_span_device(OpusMSDecoder **st, int n, int F, const unsigned char *d_data, const int64_t *d_offs,
+                                        const opus_int32 *d_len, opus_int16 *d_pcm, int frame_size, int *d_ret) {
+    if (!st || n <= 0 || F <= 0 || frame_size <= 0) return OPUS_BAD_ARG;
+    std::lock_guard<std::mutex> lk(g.mu);
+    return ms_decode_span_locked(st, n, F, d_data, 0, d_offs, d_len, d_pcm, frame_size, 0, d_ret, true, true);
+}
+
+int opus_multistream_decoder_sync(OpusMSDecoder **st, int n) {
+    if (!st || n <= 0) return OPUS_BAD_ARG;
+    std::vector<OpusDecoder *> el;
+    for (int m = 0; m < n; m++) {
+        if (!st[m] || st[m]->magic != kMsDecMagic) return OPUS_BAD_ARG;
+        for (int s = 0; s < st[m]->streams; s++) el.push_back(ms_stream(st[m], s));
+    }
+    std::lock_guard<std::mutex> lk(g.mu);
+    if (!ctx_init_locked()) return OPUS_INTERNAL_ERROR;
+    return sync_states_locked(el.data(), (int)el.size(), true);
+}
+
+// Scalar call = span of one; the embedded blocks are left current (write-back) so the decoder stays memcpy-able.
+int opus_multistream_decode(OpusMSDecoder *st, const unsigned char *data, opus_int32 len, opus_int16 *pcm, int frame_size, int decode_fec) {
+    if (frame_size <= 0) return OPUS_BAD_ARG;
+    if (!st || st->magic != kMsDecMagic || !pcm) return OPUS_BAD_ARG;
+    if (decode_fec < 0 || decode_fec > 1) return OPUS_BAD_ARG;
+    if (data == nullptr) len = 0;   // a NULL packet is a lost packet
+    if (len < 0) return OPUS_BAD_ARG;
+    // a row of the clamped size holds whatever the call can return (ms_decode_span_locked: at most 120 ms)
+    const int cap = frame_size < st->Fs / 25 * 3 ? frame_size : st->Fs / 25 * 3;
+    std::lock_guard<std::mutex> lk(g.mu);
+    std::vector<int16_t> out((size_t)cap * st->channels);
+    int64_t off = 0;
+    int32_t l = len;
+    int r = 0;
+    OpusMSDecoder *one = st;
+    const int rc = ms_decode_span_locked(&one, 1, 1, data, l, &off, &l, out.data(), cap, decode_fec, &r, false, false);
+    if (rc != OPUS_OK) return rc;
+    if (r > 0) memcpy(pcm, out.data(), (size_t)r * st->channels * sizeof(int16_t));
     return r;
 }
 

@@ -147,4 +147,37 @@ CB_HD int pkt_parse(const uint8_t *data, int len, int self_delimited, uint8_t *o
     return count;
 }
 
+// A frame length as a packet header writes it (one or two bytes; the read side is pkt_parse_size).
+CB_HD int pkt_put_size(int size, uint8_t *p) {
+    if (size < 252) {
+        p[0] = (uint8_t)size;
+        return 1;
+    }
+    p[0] = (uint8_t)(252 + (size & 3));
+    p[1] = (uint8_t)((size - p[0]) >> 2);
+    return 2;
+}
+
+// The header of an undelimited packet of `count` frames with frame-count code `code` (RFC 6716 §3.2): the TOC (configuration
+// `cfg` = TOC & 0xFC), for code 2 the first frame's length, for code 3 the frame-count byte, `pad` bytes of padding as its
+// length bytes (the padding itself follows the frames) and, VBR, the lengths of all frames but the last.  Returns its size
+// (at most 2 + 47 * 2 + (pad + 253) / 255 bytes).
+CB_HD int pkt_write_header(uint8_t *p, uint8_t cfg, int code, int count, int vbr, int pad, const int16_t *len) {
+    uint8_t *q = p;
+    *q++ = (uint8_t)(cfg | code);
+    if (code == 2) {
+        q += pkt_put_size(len[0], q);
+    } else if (code == 3) {
+        *q++ = (uint8_t)(count | (vbr ? 0x80 : 0) | (pad ? 0x40 : 0));
+        if (pad) {
+            const int n255 = (pad - 1) / 255;
+            for (int i = 0; i < n255; i++) *q++ = 255;
+            *q++ = (uint8_t)(pad - 255 * n255 - 1);
+        }
+        if (vbr)
+            for (int i = 0; i < count - 1; i++) q += pkt_put_size(len[i], q);
+    }
+    return (int)(q - p);
+}
+
 }  // namespace cb

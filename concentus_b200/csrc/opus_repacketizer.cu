@@ -21,17 +21,6 @@ struct OpusRepacketizer {
 
 namespace {
 
-// a frame length as it is written in a packet header (one or two bytes, src/opus.c:148-167 read side)
-inline int put_size(int size, unsigned char *p) {
-    if (size < 252) {
-        p[0] = (unsigned char)size;
-        return 1;
-    }
-    p[0] = (unsigned char)(252 + (size & 3));
-    p[1] = (unsigned char)((size - p[0]) >> 2);
-    return 2;
-}
-
 // How frames [begin, end) are laid out: the cheapest code that can carry them (0: one frame, 1: two equal, 2: two different,
 // 3: any count, CBR or VBR) — code 3 is forced when padding is wanted and there is room for it.
 struct Layout {
@@ -78,21 +67,7 @@ opus_int32 emit_range(const OpusRepacketizer *rp, int begin, int end, unsigned c
     const int rc = plan_layout(len, count, maxlen, want_pad, L);
     if (rc != OPUS_OK) return rc;
     unsigned char *p = data;
-    const unsigned char cfg = (unsigned char)(rp->toc & 0xFC);
-    if (L.code < 3) {
-        *p++ = (unsigned char)(cfg | L.code);
-        if (L.code == 2) p += put_size(len[0], p);
-    } else {
-        *p++ = (unsigned char)(cfg | 3);
-        *p++ = (unsigned char)(count | (L.vbr ? 0x80 : 0) | (L.pad ? 0x40 : 0));
-        if (L.pad) {
-            const int n255 = (L.pad - 1) / 255;
-            for (int i = 0; i < n255; i++) *p++ = 255;
-            *p++ = (unsigned char)(L.pad - 255 * n255 - 1);
-        }
-        if (L.vbr)
-            for (int i = 0; i < count - 1; i++) p += put_size(len[i], p);
-    }
+    p += cb::pkt_write_header(p, (unsigned char)(rp->toc & 0xFC), L.code, count, L.vbr, L.pad, len);
     for (int i = 0; i < count; i++) {
         memmove(p, frames[i], (size_t)len[i]);
         p += len[i];

@@ -227,6 +227,38 @@ int opus_encode_span_ranges(OpusEncoder **st, int n, int F, const opus_int16 *pc
                             opus_int32 max_data_bytes, opus_int32 *ret, opus_uint32 *final_range);
 int opus_encoder_sync(OpusEncoder **st, int n);
 
+/* ---- multistream decoder: libopus opus_multistream.h (opus_multistream_decoder_*), packet format RFC 6716 Appendix B, channel
+ * mapping RFC 7845 section 5.1.1.  `streams` Opus streams, the first `coupled_streams` stereo and the rest mono; coupled stream s
+ * decodes stream channels 2s and 2s+1, mono stream s stream channel coupled_streams + s; output channel c is a copy of stream channel
+ * mapping[c], or silence when mapping[c] == 255.  Streams 0..streams-2 of a packet are self-delimited, the last one takes the
+ * remaining bytes.  A packet is validated whole before any stream is decoded, so a rejected packet leaves every stream untouched;
+ * a SILK or hybrid sub-packet that carries a frame is OPUS_UNIMPLEMENTED like in opus_decode. ---- */
+typedef struct OpusMSDecoder OpusMSDecoder;
+#define OPUS_MULTISTREAM_GET_DECODER_STATE_REQUEST 5122
+#define __opus_check_decstate_ptr(ptr) ((ptr) + ((ptr) - (OpusDecoder **)(ptr)))
+#define OPUS_MULTISTREAM_GET_DECODER_STATE(x, y) OPUS_MULTISTREAM_GET_DECODER_STATE_REQUEST, __opus_check_int(x), __opus_check_decstate_ptr(y)
+opus_int32 opus_multistream_decoder_get_size(int streams, int coupled_streams);
+OpusMSDecoder *opus_multistream_decoder_create(opus_int32 Fs, int channels, int streams, int coupled_streams, const unsigned char *mapping,
+                                               int *error);
+int opus_multistream_decoder_init(OpusMSDecoder *st, opus_int32 Fs, int channels, int streams, int coupled_streams,
+                                  const unsigned char *mapping);
+int opus_multistream_decode(OpusMSDecoder *st, const unsigned char *data, opus_int32 len, opus_int16 *pcm, int frame_size, int decode_fec);
+/* OPUS_RESET_STATE and OPUS_SET_GAIN go to every stream; OPUS_GET_BANDWIDTH, _SAMPLE_RATE, _GAIN and _LAST_PACKET_DURATION are
+ * answered by stream 0; OPUS_GET_FINAL_RANGE is the XOR of all streams' final ranges; OPUS_MULTISTREAM_GET_DECODER_STATE(id, &dec)
+ * gives the embedded OpusDecoder of stream id, on which opus_decoder_ctl works. */
+int opus_multistream_decoder_ctl(OpusMSDecoder *st, int request, ...);
+void opus_multistream_decoder_destroy(OpusMSDecoder *st);
+
+/* Multistream spans (ours), the contracts of opus_decode_span / _span_device / opus_decoder_sync: multistream packet (m,f) at
+ * data[offs[m*F+f] .. +len[m*F+f]), its PCM at pcm + (m*F+f)*frame_size*channels, ret[m*F+f] what opus_multistream_decode returns.
+ * Every decoder of a span shares Fs, channels, streams and coupled_streams; mappings may differ.  Packets that overlap must do so
+ * whole (the same bytes at the same offset). */
+int opus_multistream_decode_span(OpusMSDecoder **st, int n, int F, const unsigned char *data, const int64_t *offs, const opus_int32 *len,
+                                 opus_int16 *pcm, int frame_size, int *ret);
+int opus_multistream_decode_span_device(OpusMSDecoder **st, int n, int F, const unsigned char *d_data, const int64_t *d_offs,
+                                        const opus_int32 *d_len, opus_int16 *d_pcm, int frame_size, int *d_ret);
+int opus_multistream_decoder_sync(OpusMSDecoder **st, int n);
+
 /* ---- runtime ---- */
 int opus_b200_init(int device);            /* select the CUDA device (default 0); 0 or OPUS_INTERNAL_ERROR */
 int opus_b200_synchronize(void);
@@ -234,6 +266,8 @@ void *opus_b200_stream(void);              /* the cudaStream_t the library launc
 long long opus_b200_kernel_launches(void); /* number of codec kernels launched so far by this process */
 /* Accumulated device time per pipeline stage (0 parse, 1 synth, 2 de-emphasis) in ms and launches, since the last reset. */
 int opus_b200_stage_times(double ms[3], long long launches[3], int reset);
+/* The same for the two stages of multistream calls (0 split, 1 gather). */
+int opus_b200_ms_stage_times(double ms[2], long long launches[2], int reset);
 /* Time of the last span call in milliseconds, from CUDA events recorded around it on the library stream. */
 float opus_b200_last_kernel_ms(void);
 int opus_b200_device_index(void);         /* device in use, -1 when CUDA is unusable */
