@@ -31,6 +31,8 @@ OPUS_SET_GAIN_REQUEST = 4034
 OPUS_GET_GAIN_REQUEST = 4045
 OPUS_GET_LAST_PACKET_DURATION_REQUEST = 4039
 OPUS_MULTISTREAM_GET_DECODER_STATE_REQUEST = 5122
+OPUS_MULTISTREAM_GET_ENCODER_STATE_REQUEST = 5120
+OPUS_GET_BITRATE_REQUEST = 4003
 
 _lib = None
 
@@ -50,6 +52,10 @@ EXPORTS = [
     "opus_multistream_decoder_get_size", "opus_multistream_decoder_create", "opus_multistream_decoder_init", "opus_multistream_decode",
     "opus_multistream_decoder_ctl", "opus_multistream_decoder_destroy", "opus_multistream_decode_span",
     "opus_multistream_decode_span_device", "opus_multistream_decoder_sync", "opus_b200_ms_stage_times",
+    "opus_multistream_encoder_get_size", "opus_multistream_encoder_create", "opus_multistream_encoder_init", "opus_multistream_encode",
+    "opus_multistream_encoder_ctl", "opus_multistream_encoder_destroy", "opus_multistream_surround_encoder_get_size",
+    "opus_multistream_surround_encoder_create", "opus_multistream_surround_encoder_init", "opus_multistream_encode_span",
+    "opus_multistream_encode_span_device", "opus_multistream_encoder_sync", "opus_b200_ms_enc_stage_times",
 ]
 
 OPUS_APPLICATION_VOIP = 2048
@@ -117,6 +123,23 @@ def lib():
         L.opus_multistream_decode_span_device.argtypes = L.opus_decode_span.argtypes
         L.opus_multistream_decoder_sync.argtypes = [C.c_void_p, C.c_int]
         L.opus_b200_ms_stage_times.argtypes = [C.c_void_p, C.c_void_p, C.c_int]
+        L.opus_multistream_encoder_create.restype = C.c_void_p
+        L.opus_multistream_encoder_create.argtypes = [C.c_int32, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_int, C.POINTER(C.c_int)]
+        L.opus_multistream_encoder_init.argtypes = [C.c_void_p, C.c_int32, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_int]
+        L.opus_multistream_encoder_get_size.argtypes = [C.c_int, C.c_int]
+        L.opus_multistream_surround_encoder_get_size.argtypes = [C.c_int, C.c_int]
+        L.opus_multistream_surround_encoder_create.restype = C.c_void_p
+        L.opus_multistream_surround_encoder_create.argtypes = [C.c_int32, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int,
+                                                               C.POINTER(C.c_int)]
+        L.opus_multistream_surround_encoder_init.argtypes = [C.c_void_p, C.c_int32, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p,
+                                                             C.c_int]
+        L.opus_multistream_encoder_destroy.argtypes = [C.c_void_p]
+        L.opus_multistream_encoder_destroy.restype = None
+        L.opus_multistream_encode.argtypes = L.opus_encode.argtypes
+        L.opus_multistream_encode_span.argtypes = L.opus_encode_span.argtypes
+        L.opus_multistream_encode_span_device.argtypes = L.opus_encode_span.argtypes
+        L.opus_multistream_encoder_sync.argtypes = [C.c_void_p, C.c_int]
+        L.opus_b200_ms_enc_stage_times.argtypes = [C.c_void_p, C.c_void_p, C.c_int]
         _lib = L
     return _lib
 
@@ -219,6 +242,78 @@ class MSDecoderBatch:
         for i in range(self.n):
             if self.handles[i]:
                 L.opus_multistream_decoder_destroy(C.c_void_p(self.handles[i]))
+                self.handles[i] = None
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+
+class MSEncoderBatch:
+    """n multistream encoders (same Fs / channels / streams / coupled streams) driven through the multistream span C ABI.
+    mapping: one channel mapping for all encoders, or one per encoder.  bitrate is the multistream bitrate; vbr / cvbr /
+    complexity go to every stream."""
+
+    def __init__(self, n, Fs, channels, streams, coupled, mapping, application=OPUS_APPLICATION_RESTRICTED_LOWDELAY, bitrate=OPUS_AUTO,
+                 vbr=1, cvbr=1, complexity=9):
+        L = lib()
+        self.n, self.Fs, self.channels, self.streams, self.coupled = n, Fs, channels, streams, coupled
+        maps = np.asarray(mapping, dtype=np.uint8).reshape(-1, channels)
+        if maps.shape[0] == 1:
+            maps = np.repeat(maps, n, axis=0)
+        assert maps.shape[0] == n
+        self.mappings = np.ascontiguousarray(maps)
+        err = C.c_int(0)
+        self.handles = (C.c_void_p * n)()
+        for i in range(n):
+            h = L.opus_multistream_encoder_create(Fs, channels, streams, coupled, _p(self.mappings[i]), application, C.byref(err))
+            if not h:
+                raise RuntimeError("opus_multistream_encoder_create failed: %d" % err.value)
+            self.handles[i] = h
+            for req, v in ((OPUS_SET_BITRATE_REQUEST, bitrate), (OPUS_SET_VBR_REQUEST, vbr), (OPUS_SET_VBR_CONSTRAINT_REQUEST, cvbr),
+                           (OPUS_SET_COMPLEXITY_REQUEST, complexity)):
+                rc = L.opus_multistream_encoder_ctl(C.c_void_p(h), req, C.c_int32(v))
+                if rc != OPUS_OK:
+                    raise RuntimeError("opus_multistream_encoder_ctl(%d, %d) -> %d" % (req, v, rc))
+
+    def encode_span(self, pcm, F, frame_size, max_data_bytes):
+        """pcm: int16 [n*F*frame_size, channels] (encoder-major).  Returns (data uint8 [n*F, max_data_bytes], rets int32 [n*F])."""
+        L = lib()
+        pcm = np.ascontiguousarray(pcm, dtype=np.int16)
+        assert pcm.size == self.n * F * frame_size * self.channels
+        data = np.zeros((self.n * F, max_data_bytes), dtype=np.uint8)
+        rets = np.zeros(self.n * F, dtype=np.int32)
+        rc = L.opus_multistream_encode_span(self.handles, self.n, F, _p(pcm), frame_size, _p(data), max_data_bytes, _p(rets))
+        if rc != OPUS_OK:
+            raise RuntimeError("opus_multistream_encode_span: %s" % L.opus_strerror(rc).decode())
+        return data, rets
+
+    def _get(self, request):
+        L = lib()
+        out = np.zeros(self.n, dtype=np.uint32 if request == OPUS_GET_FINAL_RANGE_REQUEST else np.int32)
+        v = C.c_int32(0)
+        for i in range(self.n):
+            rc = L.opus_multistream_encoder_ctl(C.c_void_p(self.handles[i]), request, C.byref(v))
+            if rc != OPUS_OK:
+                raise RuntimeError("opus_multistream_encoder_ctl(%d) -> %d" % (request, rc))
+            out[i] = v.value & 0xFFFFFFFF if request == OPUS_GET_FINAL_RANGE_REQUEST else v.value
+        return out
+
+    def final_ranges(self):
+        """OPUS_GET_FINAL_RANGE of each multistream encoder: the XOR of its streams' final ranges."""
+        return self._get(OPUS_GET_FINAL_RANGE_REQUEST)
+
+    def bitrates(self):
+        """OPUS_GET_BITRATE of each multistream encoder: the sum of its streams' bitrates."""
+        return self._get(OPUS_GET_BITRATE_REQUEST)
+
+    def close(self):
+        L = lib()
+        for i in range(self.n):
+            if self.handles[i]:
+                L.opus_multistream_encoder_destroy(C.c_void_p(self.handles[i]))
                 self.handles[i] = None
 
     def __del__(self):

@@ -1,9 +1,10 @@
-// opus_multistream.h — the packet side of the multistream decoder, usable from host and device code.
+// opus_multistream.h — the packet side of the multistream decoder and encoder, usable from host and device code.
 //
 // A multistream packet of S streams (RFC 7845 §5.1.1, libopus opus_multistream.h) carries one Opus packet per stream: streams
 // 0..S-2 in self-delimited framing (RFC 6716 Appendix B), the last stream as an ordinary packet made of all remaining bytes.
 // ms_split_packet validates such a packet the way opus_multistream_decode does before it decodes anything, and rewrites it as S
-// ordinary packets that the single-stream decoder stages take unchanged.
+// ordinary packets that the single-stream decoder stages take unchanged.  ms_pack_packet is the encoder's inverse: it frames one
+// stream's ordinary packet for its place in a multistream packet.
 #pragma once
 #include "opus_packet.h"
 
@@ -89,6 +90,31 @@ CB_HD int ms_split_packet(const uint8_t *data, int len, int S, int Fs, int frame
         elens[s * estride] = ret < 0 ? kMsRejectLen : 0;
     }
     return ret;
+}
+
+// The encoder's side: stream s's ordinary packet pkt[0..len) as it goes into a multistream packet, written to out[0..maxlen)
+// (which must not overlap pkt).  This is opus_repacketizer_cat followed by opus_repacketizer_out_range_impl over all its frames
+// (repacketizer.c:62-227): the frames are re-framed with the cheapest frame-count code (plan_layout), the packet's own padding
+// is dropped, streams 0..S-2 are self-delimited (RFC 6716 Appendix B) and with `pad` (the last stream of a CBR call) the packet
+// is padded to exactly maxlen.  Returns the bytes written or a negative error (the packet's parse error, OPUS_BUFFER_TOO_SMALL).
+CB_HD int ms_pack_packet(const uint8_t *pkt, int len, int self_delimited, int pad, uint8_t *out, int maxlen) {
+    int16_t size[48];
+    uint8_t toc;
+    int poff = 0;
+    const int count = pkt_parse(pkt, len, 0, &toc, size, &poff, nullptr);
+    if (count < 0) return count;
+    const int sd = self_delimited ? 1 + (size[count - 1] >= 252) : 0;
+    PktLayout L;
+    const int rc = plan_layout(size, count, maxlen, pad, L, sd);
+    if (rc < 0) return rc;
+    uint8_t *q = out + pkt_write_header(out, (uint8_t)(toc & 0xFC), L.code, count, L.vbr, L.pad, size);
+    if (self_delimited) q += pkt_put_size(size[count - 1], q);
+    const uint8_t *src = pkt + poff;
+    int payload = 0;
+    for (int i = 0; i < count; i++) payload += size[i];
+    for (int i = 0; i < payload; i++) *q++ = src[i];
+    while (q < out + L.total) *q++ = 0;   // the padding bytes
+    return L.total;
 }
 
 }  // namespace cb

@@ -180,4 +180,42 @@ CB_HD int pkt_write_header(uint8_t *p, uint8_t cfg, int code, int count, int vbr
     return (int)(q - p);
 }
 
+// How `count` frames of lengths len[] are laid out by opus_repacketizer_out_range_impl (repacketizer.c:102-227): the cheapest code
+// that can carry them (0: one frame, 1: two equal, 2: two different, 3: any count, CBR or VBR) — code 3 is forced when padding is
+// wanted and there is room for it.  `sd` is the size of a self-delimiting length (0 for an ordinary packet, else 1 or 2 bytes for
+// the last frame's length), which counts towards header and total.  Returns 0 or OPUS_BUFFER_TOO_SMALL when the packet exceeds
+// maxlen; with want_pad the packet is padded to exactly maxlen (pad includes the padding-length bytes themselves).
+struct PktLayout {
+    int code, vbr, header, total, pad;
+};
+CB_HD int plan_layout(const int16_t *len, int count, int maxlen, int want_pad, PktLayout &L, int sd = 0) {
+    int payload = 0;
+    for (int i = 0; i < count; i++) payload += len[i];
+    L.pad = 0;
+    L.vbr = 0;
+    if (count == 1) { L.code = 0; L.header = 1; }
+    else if (count == 2 && len[0] == len[1]) { L.code = 1; L.header = 1; }
+    else if (count == 2) { L.code = 2; L.header = 1 + 1 + (len[0] >= 252); }
+    else L.code = 3;
+    if (L.code != 3) {
+        L.header += sd;
+        L.total = L.header + payload;
+        if (L.total > maxlen) return -2;   // OPUS_BUFFER_TOO_SMALL
+        if (!(want_pad && L.total < maxlen)) return 0;
+        L.code = 3;   // padding needs the code-3 header
+    }
+    for (int i = 1; i < count; i++)
+        if (len[i] != len[0]) { L.vbr = 1; break; }
+    L.header = 2 + sd;
+    if (L.vbr)
+        for (int i = 0; i < count - 1; i++) L.header += 1 + (len[i] >= 252);
+    L.total = L.header + payload;
+    if (L.total > maxlen) return -2;
+    if (want_pad && L.total < maxlen) {
+        L.pad = maxlen - L.total;
+        L.total = maxlen;
+    }
+    return 0;
+}
+
 }  // namespace cb

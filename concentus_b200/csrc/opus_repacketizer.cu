@@ -21,41 +21,6 @@ struct OpusRepacketizer {
 
 namespace {
 
-// How frames [begin, end) are laid out: the cheapest code that can carry them (0: one frame, 1: two equal, 2: two different,
-// 3: any count, CBR or VBR) — code 3 is forced when padding is wanted and there is room for it.
-struct Layout {
-    int code, vbr, header, total, pad;
-};
-
-int plan_layout(const opus_int16 *len, int count, opus_int32 maxlen, int want_pad, Layout &L) {
-    int payload = 0;
-    for (int i = 0; i < count; i++) payload += len[i];
-    L.pad = 0;
-    L.vbr = 0;
-    if (count == 1) { L.code = 0; L.header = 1; }
-    else if (count == 2 && len[0] == len[1]) { L.code = 1; L.header = 1; }
-    else if (count == 2) { L.code = 2; L.header = 1 + 1 + (len[0] >= 252); }
-    else L.code = 3;
-    if (L.code != 3) {
-        L.total = L.header + payload;
-        if (L.total > maxlen) return OPUS_BUFFER_TOO_SMALL;
-        if (!(want_pad && L.total < maxlen)) return OPUS_OK;
-        L.code = 3;   // padding needs the code-3 header
-    }
-    for (int i = 1; i < count; i++)
-        if (len[i] != len[0]) { L.vbr = 1; break; }
-    L.header = 2;
-    if (L.vbr)
-        for (int i = 0; i < count - 1; i++) L.header += 1 + (len[i] >= 252);
-    L.total = L.header + payload;
-    if (L.total > maxlen) return OPUS_BUFFER_TOO_SMALL;
-    if (want_pad && L.total < maxlen) {
-        L.pad = maxlen - L.total;   // includes the padding-length bytes themselves
-        L.total = maxlen;
-    }
-    return OPUS_OK;
-}
-
 // opus_repacketizer_out_range_impl (repacketizer.c:102-227) without self-delimited framing.  `data` may overlap the frames as
 // long as every frame lies at or after the place it is moved to (in-place pad / unpad): frames are moved front to back.
 opus_int32 emit_range(const OpusRepacketizer *rp, int begin, int end, unsigned char *data, opus_int32 maxlen, int want_pad) {
@@ -63,8 +28,8 @@ opus_int32 emit_range(const OpusRepacketizer *rp, int begin, int end, unsigned c
     const int count = end - begin;
     const opus_int16 *len = rp->len + begin;
     const unsigned char *const *frames = rp->frames + begin;
-    Layout L;
-    const int rc = plan_layout(len, count, maxlen, want_pad, L);
+    cb::PktLayout L;
+    const int rc = cb::plan_layout(len, count, maxlen, want_pad, L);
     if (rc != OPUS_OK) return rc;
     unsigned char *p = data;
     p += cb::pkt_write_header(p, (unsigned char)(rp->toc & 0xFC), L.code, count, L.vbr, L.pad, len);

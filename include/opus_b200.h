@@ -259,6 +259,53 @@ int opus_multistream_decode_span_device(OpusMSDecoder **st, int n, int F, const 
                                         const opus_int32 *d_len, opus_int16 *d_pcm, int frame_size, int *d_ret);
 int opus_multistream_decoder_sync(OpusMSDecoder **st, int n);
 
+/* ---- multistream encoder: libopus opus_multistream.h (opus_multistream_encoder_*, opus_multistream_surround_encoder_*), the
+ * packet format of the multistream decoder above.  Input channel c feeds stream channel mapping[c] (255: the channel is ignored);
+ * a stream channel fed by several input channels takes the first of them.  Every coupled stream needs both of its channels and
+ * every mono stream its channel, else init is OPUS_BAD_ARG.  Each call gives every stream its share of the multistream bitrate
+ * (libopus's surround_rate_allocation without an LFE stream) and codes the streams in order, each within the bytes the earlier
+ * ones left (at most 1276 per stream, the single-stream clamp of opus_encode); in CBR the last stream is padded to fill the packet.
+ * A stream that fails ends the call with its error: the streams before it have advanced, those after it are untouched.
+ * Surround masking and LFE streams are not built: the surround encoder takes mapping families 0 and 1 with 1-2 channels and
+ * family 255, and returns OPUS_UNIMPLEMENTED for family 1 with 3-8 channels.  A 5.1 stream can still be written with the explicit
+ * layout (streams 4, coupled 2, mapping {0,4,1,2,3,5}); it is a valid family-1 stream, not the one libopus's surround encoder
+ * would write. ---- */
+typedef struct OpusMSEncoder OpusMSEncoder;
+#define OPUS_MULTISTREAM_GET_ENCODER_STATE_REQUEST 5120
+#define __opus_check_encstate_ptr(ptr) ((ptr) + ((ptr) - (OpusEncoder **)(ptr)))
+#define OPUS_MULTISTREAM_GET_ENCODER_STATE(x, y) OPUS_MULTISTREAM_GET_ENCODER_STATE_REQUEST, __opus_check_int(x), __opus_check_encstate_ptr(y)
+/* The size of this library's block: a header and `streams` OpusEncoder blocks (not libopus's size). */
+opus_int32 opus_multistream_encoder_get_size(int streams, int coupled_streams);
+opus_int32 opus_multistream_surround_encoder_get_size(int channels, int mapping_family);
+OpusMSEncoder *opus_multistream_encoder_create(opus_int32 Fs, int channels, int streams, int coupled_streams, const unsigned char *mapping,
+                                               int application, int *error);
+OpusMSEncoder *opus_multistream_surround_encoder_create(opus_int32 Fs, int channels, int mapping_family, int *streams, int *coupled_streams,
+                                                        unsigned char *mapping, int application, int *error);
+int opus_multistream_encoder_init(OpusMSEncoder *st, opus_int32 Fs, int channels, int streams, int coupled_streams, const unsigned char *mapping,
+                                  int application);
+int opus_multistream_surround_encoder_init(OpusMSEncoder *st, opus_int32 Fs, int channels, int mapping_family, int *streams, int *coupled_streams,
+                                           unsigned char *mapping, int application);
+/* Returns the packet length or an error: OPUS_BAD_ARG for a frame size no stream codes, OPUS_BUFFER_TOO_SMALL when
+ * max_data_bytes < 4*streams - 1. */
+opus_int32 opus_multistream_encode(OpusMSEncoder *st, const opus_int16 *pcm, int frame_size, unsigned char *data, opus_int32 max_data_bytes);
+/* OPUS_SET_BITRATE sets the multistream bitrate (OPUS_AUTO, OPUS_BITRATE_MAX or >= 0, not clamped); OPUS_GET_BITRATE is the sum of
+ * the streams' bitrates and OPUS_GET_FINAL_RANGE the XOR of their final ranges; OPUS_RESET_STATE and the other SETs go to every
+ * stream, the other GETs are answered by stream 0; OPUS_MULTISTREAM_GET_ENCODER_STATE(id, &enc) gives the embedded OpusEncoder of
+ * stream id, on which opus_encoder_ctl works. */
+int opus_multistream_encoder_ctl(OpusMSEncoder *st, int request, ...);
+void opus_multistream_encoder_destroy(OpusMSEncoder *st);
+
+/* Multistream encode spans (ours), the contracts of opus_encode_span / _span_device / opus_encoder_sync: PCM of frame (m,f) at
+ * pcm + (m*F+f)*frame_size*channels, its packet at data + (m*F+f)*max_data_bytes, ret[m*F+f] what opus_multistream_encode returns.
+ * Every encoder of a span shares Fs, channels, streams and coupled_streams; mappings and settings may differ.  _device: pcm / data /
+ * ret are DEVICE pointers and the call only enqueues on the encoder stream (except in CBR, where it waits for the call to read the
+ * last stream's final bitrate back); opus_b200_enc_synchronize() waits. */
+int opus_multistream_encode_span(OpusMSEncoder **st, int n, int F, const opus_int16 *pcm, int frame_size, unsigned char *data,
+                                 opus_int32 max_data_bytes, opus_int32 *ret);
+int opus_multistream_encode_span_device(OpusMSEncoder **st, int n, int F, const opus_int16 *d_pcm, int frame_size, unsigned char *d_data,
+                                        opus_int32 max_data_bytes, opus_int32 *d_ret);
+int opus_multistream_encoder_sync(OpusMSEncoder **st, int n);
+
 /* ---- runtime ---- */
 int opus_b200_init(int device);            /* select the CUDA device (default 0); 0 or OPUS_INTERNAL_ERROR */
 int opus_b200_synchronize(void);
@@ -268,6 +315,8 @@ long long opus_b200_kernel_launches(void); /* number of codec kernels launched s
 int opus_b200_stage_times(double ms[3], long long launches[3], int reset);
 /* The same for the two stages of multistream calls (0 split, 1 gather). */
 int opus_b200_ms_stage_times(double ms[2], long long launches[2], int reset);
+/* The same for the multistream encoder's kernels (0 route, 1 budget, 2 pack), on the encoder stream. */
+int opus_b200_ms_enc_stage_times(double ms[3], long long launches[3], int reset);
 /* Time of the last span call in milliseconds, from CUDA events recorded around it on the library stream. */
 float opus_b200_last_kernel_ms(void);
 int opus_b200_device_index(void);         /* device in use, -1 when CUDA is unusable */
