@@ -220,4 +220,14 @@ CB_DEV unsigned lcg_jump(unsigned seed, int k) { return kLcgMul[k] * seed + kLcg
 CB_DEV unsigned udiv(unsigned n, unsigned d) { return n / d; }
 CB_DEV int sudiv(int n, int d) { return n / d; }
 
+// Division of team-loop indices by a divisor fixed for the loop: n / d == umulhi(n, fastdiv_magic(d)) exactly whenever
+// 2 <= d and n * d < 2^32 (the rounding error of the magic is below 1/d).  One multiply-high per item instead of the
+// dozen-instruction sequence of a division by a runtime value; the magic itself is one division per loop.
+CB_DEV unsigned fastdiv_magic(unsigned d) { return 0xffffffffu / d + 1u; }
+#if defined(__CUDACC__)
+CB_DEV int fastdiv(int n, unsigned magic) { return (int)__umulhi((unsigned)n, magic); }
+#else
+CB_DEV int fastdiv(int n, unsigned magic) { return (int)(((uint64_t)(unsigned)n * magic) >> 32); }
+#endif
+
 }  // namespace cb

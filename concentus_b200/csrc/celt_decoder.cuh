@@ -133,18 +133,25 @@ CB_DEV void celt_parse_frame(const uint8_t *data, int len, int LM, int C, int en
 // Stage B
 // ---------------------------------------------------------------------------------------------------
 
-// Team-shared working set of one frame synthesis (~4.1 KB).
+enum { kDenBins = 100 };   // eBands[nbEBands]: bins of the coded bands at LM = 0
+
+// Team-shared working set of one frame synthesis (~4.8 KB).
 struct SynthScratch {
     int fft[kMaxFrame];                               // IMDCT buffer
     int16_t den_gain[2][kNbEBands];                   // denormalisation gain / shift per band
     int8_t den_shift[2][kNbEBands];
+    // denormalisation per bin at LM = 0 resolution (bin j of the frame reads den[c][j >> LM]): (G << 5) | R, where
+    // X[j] * G >> R equals the reference's gain product and shift (0 outside the decoded bands)
+    int den[2][kDenBins];
 };
 
 // comb_filter with y == x (celt/celt.c:183-244, as called at celt_decoder.c:1002-1013).  In place the
 // filter is recursive: output i reads positions <= i-T+2, already final.  Outputs within a run of
-// min(T0,T1)-2 (>= 13) samples are mutually independent, so runs are spread over the lanes.
+// min(T0,T1)-2 (>= 13) samples are mutually independent, so runs are spread over the lanes.  Every sample it changes is
+// also stored to y[i] when y is given.
 template <class TM>
-CB_DEV void comb_filter_inplace(TM tm, int *x, int T0, int T1, int N, int g0, int g1, int tapset0, int tapset1, int overlap) {
+CB_DEV void comb_filter_inplace(TM tm, int *x, int T0, int T1, int N, int g0, int g1, int tapset0, int tapset1, int overlap,
+                                int *y = nullptr) {
     if (g0 == 0 && g1 == 0) return;
     const int g00 = s16(mul16_16_p15(g0, kCombGains[tapset0][0]));
     const int g01 = s16(mul16_16_p15(g0, kCombGains[tapset0][1]));
@@ -174,6 +181,7 @@ CB_DEV void comb_filter_inplace(TM tm, int *x, int T0, int T1, int N, int g0, in
                 v = wadd(v, mul16_32_q15(mul16_16_q15(f, g12), wadd(x[i - T1 + 2], x[i - T1 - 2])));
             }
             x[i] = v;
+            if (y) y[i] = v;
         }
         tm.sync();
     }
@@ -186,6 +194,7 @@ CB_DEV void comb_filter_inplace(TM tm, int *x, int T0, int T1, int N, int g0, in
             v = wadd(v, mul16_32_q15(g11, wadd(x[i - T1 + 1], x[i - T1 - 1])));
             v = wadd(v, mul16_32_q15(g12, wadd(x[i - T1 + 2], x[i - T1 - 2])));
             x[i] = v;
+            if (y) y[i] = v;
         }
         tm.sync();
     }
@@ -272,57 +281,60 @@ CB_DEV void history_shift(TM tm, int *mem, int N, int count = -1) {
 }
 
 // celt_synthesis (celt_decoder.c:280-350) with denormalise_bands (bands.c:169-238) fused into the IMDCT pre-rotation.
-// X: C*N normalised spectrum; out_syn[c]: synthesis target (tail of the channel's history).
+// X: C*N normalised spectrum; out_syn[c]: synthesis target (tail of the channel's history).  When sig is given, the
+// frame's N output samples of channel c are also stored to sig[c].
 template <class TM>
 CB_DEV void celt_synthesis_team(TM tm, SynthScratch &S, const int16_t *X, int *const *out_syn, const int16_t *oldBandE, int start, int effEnd,
-                                int C, int CC, int isTransient, int LM, int downsample, int silence) {
+                                int C, int CC, int isTransient, int LM, int downsample, int silence, int *const *sig = nullptr) {
     const int M = 1 << LM;
     const int N = M * kShortMdct;
-    {
-        int bstart = start, bend = effEnd;
-        int bound = M * kEBands[bend];
-        if (downsample != 1) bound = imin(bound, N / downsample);
-        if (silence) { bound = 0; bstart = bend = 0; }
-        const int lo = M * kEBands[bstart];
-        CB_TEAM_FOR(w, C * kNbEBands, tm) {   // per-band gain/shift (bands.c:195-227)
-            int c = w / kNbEBands, i = w - c * kNbEBands;
-            int lg = s16(oldBandE[c * kNbEBands + i] + shl16(kEMeans[i], 6));
-            int shift = 16 - (lg >> 10);
-            int g;
-            if (shift > 31) { shift = 0; g = 0; }
-            else g = celt_exp2_frac(lg & 1023);
-            if (shift < -2) { g = 32767; shift = -2; }
-            S.den_gain[c][i] = (int16_t)g;
-            S.den_shift[c][i] = (int8_t)shift;
+    int bstart = start, bend = effEnd;
+    int bound = M * kEBands[bend];
+    if (downsample != 1) bound = imin(bound, N / downsample);
+    if (silence) { bound = 0; bstart = bend = 0; }
+    CB_TEAM_FOR(w, C * kNbEBands, tm) {   // per-band gain/shift (bands.c:195-227)
+        int c = w / kNbEBands, i = w - c * kNbEBands;
+        int lg = s16(oldBandE[c * kNbEBands + i] + shl16(kEMeans[i], 6));
+        int shift = 16 - (lg >> 10);
+        int g;
+        if (shift > 31) { shift = 0; g = 0; }
+        else g = celt_exp2_frac(lg & 1023);
+        if (shift < -2) { g = 32767; shift = -2; }
+        S.den_gain[c][i] = (int16_t)g;
+        S.den_shift[c][i] = (int8_t)shift;
+    }
+    tm.sync();
+    // Spread over the bins, with the shift folded into the gain: for shift < 0, (X*g) << -shift == X*(g << -shift)
+    // mod 2^32, so each bin costs one multiply and one right shift, without a band look-up or a branch.
+    CB_TEAM_FOR(w, C * kDenBins, tm) {
+        const int c = w >= kDenBins, k = w - c * kDenBins;
+        const int b = kBinToBand[k];
+        int e = 0;
+        if (b >= bstart && b < bend) {
+            const int sh = S.den_shift[c][b];
+            e = ((int)S.den_gain[c][b] << (imax(-sh, 0) + 5)) | imax(sh, 0);
         }
-        tm.sync();
-        const int B = isTransient ? M : 1;
-        const int shift = isTransient ? kMaxLM : kMaxLM - LM;
-        const int hi = imin(bound, M * kEBands[bend]);
-        // mode 0: channel 0; 1: channel 1; 2: (ch0+ch1)/2 downmix (celt_decoder.c:325-339)
-        auto freq = [&](int mode, int j) -> int {
-            if (j < lo || j >= hi) return 0;
-            const int b = kBinToBand[j >> LM];
-            int v0 = 0, v1 = 0;
-            if (mode != 1) {
-                int v = mul16_16(X[j], S.den_gain[0][b]);
-                int sh = S.den_shift[0][b];
-                v0 = sh < 0 ? shl32(v, -sh) : (v >> sh);
-            }
-            if (mode != 0) {
-                int v = mul16_16(X[N + j], S.den_gain[1][b]);
-                int sh = S.den_shift[1][b];
-                v1 = sh < 0 ? shl32(v, -sh) : (v >> sh);
-            }
-            return mode == 0 ? v0 : mode == 1 ? v1 : (wadd(v0, v1) >> 1);
-        };
-        const int npass = (CC == 2 && C == 2) ? 2 : 1;
-        CB_NOUNROLL for (int p = 0; p < npass; p++) {
-            const int mode = (CC == 1 && C == 2) ? 2 : p;
-            imdct_compute(tm, [&](int j) { return freq(mode, j); }, B, shift, S.fft);
-            imdct_assemble(tm, out_syn[p], B, shift, S.fft);
-            if (CC == 2 && C == 1) imdct_assemble(tm, out_syn[1], B, shift, S.fft);   // mono stream into two channels
-        }
+        S.den[c][k] = e;
+    }
+    tm.sync();
+    const int B = isTransient ? M : 1;
+    const int shift = isTransient ? kMaxLM : kMaxLM - LM;
+    const int hi = imin(bound, M * kEBands[bend]);
+    auto den = [&](int c, int j) -> int {
+        const int e = S.den[c][j >> LM];
+        return wmul(X[c * N + j], e >> 5) >> (e & 31);
+    };
+    // mode 0: channel 0; 1: channel 1; 2: (ch0+ch1)/2 downmix (celt_decoder.c:325-339)
+    auto freq = [&](int mode, int j) -> int {
+        if (j >= hi) return 0;
+        return mode != 2 ? den(mode, j) : (wadd(den(0, j), den(1, j)) >> 1);
+    };
+    const int npass = (CC == 2 && C == 2) ? 2 : 1;
+    CB_NOUNROLL for (int p = 0; p < npass; p++) {
+        const int mode = (CC == 1 && C == 2) ? 2 : p;
+        imdct_compute(tm, [&](int j) { return freq(mode, j); }, B, shift, S.fft);
+        imdct_assemble(tm, out_syn[p], B, shift, S.fft, sig ? sig[p] : nullptr);
+        if (CC == 2 && C == 1) imdct_assemble(tm, out_syn[1], B, shift, S.fft, sig ? sig[1] : nullptr);   // mono stream into two channels
     }
 }
 
@@ -344,14 +356,16 @@ CB_DEV int celt_synth_frame(TM tm, CbDecState *st, SynthScratch &S, const CbFram
     const int effEnd = imin(end, kNbEBands);
     int16_t *oldBandE = st->oldEBands, *oldLogE = st->oldLogE, *oldLogE2 = st->oldLogE2, *backgroundLogE = st->backgroundLogE;
 
-    // ---- energies: prediction recurrence is serial over bands, tiny -> lane 0 ----
+    // ---- energies: the prediction recurrence is serial over bands -> lane 0; the fine offsets are per band ----
     if (tm.lane() == 0) {
         if (C == 1)
             CB_NOUNROLL for (int i = 0; i < kNbEBands; i++) oldBandE[i] = (int16_t)imax(oldBandE[i], oldBandE[kNbEBands + i]);
         apply_coarse_energy(start, end, oldBandE, ir.qi, (ir.flags & CB_IR_INTRA) != 0, C, LM);
-        CB_NOUNROLL for (int c = 0; c < C; c++)
-            CB_NOUNROLL for (int i = start; i < end; i++)
-                oldBandE[c * kNbEBands + i] = (int16_t)(oldBandE[c * kNbEBands + i] + ir.eoff[c * kNbEBands + i]);
+    }
+    tm.sync();
+    CB_TEAM_FOR(w, C * kNbEBands, tm) {
+        const int i = w >= kNbEBands ? w - kNbEBands : w;
+        if (i >= start && i < end) oldBandE[w] = (int16_t)(oldBandE[w] + ir.eoff[w]);
     }
     tm.sync();
     CB_NOUNROLL for (int c = 0; c < CC; c++) history_shift(tm, decode_mem[c], N);
@@ -363,18 +377,19 @@ CB_DEV int celt_synth_frame(TM tm, CbDecState *st, SynthScratch &S, const CbFram
     }
 
     // ---- celt_synthesis (celt_decoder.c:280-350) with denormalise_bands (bands.c:169-238) fused in ----
-    celt_synthesis_team(tm, S, X, out_syn, oldBandE, start, effEnd, C, CC, isTransient, LM, st->downsample, silence);
+    celt_synthesis_team(tm, S, X, out_syn, oldBandE, start, effEnd, C, CC, isTransient, LM, st->downsample, silence, sig);
 
-    // ---- post-filter (celt_decoder.c:1001-1025) ----
+    // ---- post-filter (celt_decoder.c:1001-1025); what it changes is staged to sig as well ----
     const int pf_period = imax(st->postfilter_period, kCombMinPeriod);
     const int pf_period_old = imax(st->postfilter_period_old, kCombMinPeriod);
     const int postfilter_pitch = ir.pf_pitch, postfilter_gain = ir.pf_gain, postfilter_tapset = ir.pf_tapset;
+    const int max_inc = st->loss_count < 10 ? M : 1024;   // energy history, read before lane 0 resets loss_count: M*QCONST16(0.001f,DB_SHIFT) ; QCONST16(1.f,DB_SHIFT)
     CB_NOUNROLL for (int c = 0; c < CC; c++) {
         comb_filter_inplace(tm, out_syn[c], pf_period_old, pf_period, kShortMdct, st->postfilter_gain_old, st->postfilter_gain,
-                            st->postfilter_tapset_old, st->postfilter_tapset, kOverlap);
+                            st->postfilter_tapset_old, st->postfilter_tapset, kOverlap, sig[c]);
         if (LM != 0)
             comb_filter_inplace(tm, out_syn[c] + kShortMdct, pf_period, postfilter_pitch, N - kShortMdct, st->postfilter_gain,
-                                postfilter_gain, st->postfilter_tapset, postfilter_tapset, kOverlap);
+                                postfilter_gain, st->postfilter_tapset, postfilter_tapset, kOverlap, sig[c] + kShortMdct);
     }
     tm.sync();
     if (tm.lane() == 0) {
@@ -389,38 +404,29 @@ CB_DEV int celt_synth_frame(TM tm, CbDecState *st, SynthScratch &S, const CbFram
             st->postfilter_gain_old = st->postfilter_gain;
             st->postfilter_tapset_old = st->postfilter_tapset;
         }
-        // ---- energy history (celt_decoder.c:1027-1062) ----
-        if (C == 1)
-            CB_NOUNROLL for (int i = 0; i < kNbEBands; i++) oldBandE[kNbEBands + i] = oldBandE[i];
-        if (!isTransient) {
-            const int max_inc = st->loss_count < 10 ? M : 1024;   // M*QCONST16(0.001f,DB_SHIFT) ; QCONST16(1.f,DB_SHIFT)
-            CB_NOUNROLL for (int i = 0; i < 2 * kNbEBands; i++) {
-                oldLogE2[i] = oldLogE[i];
-                oldLogE[i] = oldBandE[i];
-                backgroundLogE[i] = (int16_t)imin(backgroundLogE[i] + max_inc, (int)oldBandE[i]);
-            }
-        } else {
-            CB_NOUNROLL for (int i = 0; i < 2 * kNbEBands; i++) oldLogE[i] = (int16_t)imin(oldLogE[i], oldBandE[i]);
-        }
-        CB_NOUNROLL for (int c = 0; c < 2; c++) {
-            CB_NOUNROLL for (int i = 0; i < start; i++) {
-                oldBandE[c * kNbEBands + i] = 0;
-                oldLogE[c * kNbEBands + i] = oldLogE2[c * kNbEBands + i] = -28672;
-            }
-            CB_NOUNROLL for (int i = end; i < kNbEBands; i++) {
-                oldBandE[c * kNbEBands + i] = 0;
-                oldLogE[c * kNbEBands + i] = oldLogE2[c * kNbEBands + i] = -28672;
-            }
-        }
         st->rng = ir.rng_final;
         st->loss_count = 0;
         if (ir.flags & CB_IR_EC_ERROR) st->error = 1;
     }
-    tm.sync();
-    CB_NOUNROLL for (int c = 0; c < CC; c++) {
-        const int *src = out_syn[c];
-        int *dst = sig[c];
-        CB_TEAM_FOR(j, N, tm) dst[j] = src[j];
+    // ---- energy history (celt_decoder.c:1027-1062), one band per lane ----
+    if (C == 1) {
+        CB_TEAM_FOR(i, kNbEBands, tm) oldBandE[kNbEBands + i] = oldBandE[i];
+        tm.sync();
+    }
+    CB_TEAM_FOR(w, 2 * kNbEBands, tm) {
+        const int i = w >= kNbEBands ? w - kNbEBands : w;
+        const int e = oldBandE[w];
+        if (!isTransient) {
+            oldLogE2[w] = oldLogE[w];
+            oldLogE[w] = (int16_t)e;
+            backgroundLogE[w] = (int16_t)imin(backgroundLogE[w] + max_inc, e);
+        } else {
+            oldLogE[w] = (int16_t)imin(oldLogE[w], e);
+        }
+        if (i < start || i >= end) {
+            oldBandE[w] = 0;
+            oldLogE[w] = oldLogE2[w] = -28672;
+        }
     }
     tm.sync();
     if (ir.flags & CB_IR_OVERRUN) return OPUS_INTERNAL_ERROR_;

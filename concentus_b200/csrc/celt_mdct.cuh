@@ -44,13 +44,14 @@ CB_DEV void fft_inplace(TM tm, Cpx *buf, int s, int nblocks) {
         const int mm = p * m;
         const int ngroups = nfft / mm;
         const int fs = ngroups << pl.tw_shift;   // twiddle stride (fstride<<shift)
+        // Item w = (g, j) with g = block * ngroups + group and j < m.  Blocks are nfft = ngroups * mm apart, so butterfly
+        // (g, j) starts at g * mm + j = w + g * (mm - m): one division, by m, and none by ngroups.
         if (p == 2) {
             // kf_bfly2, m == 4 (kiss_fft.c:51-108): item = (block, group, lane-in-group 0..3)
             const int items = nblocks * ngroups * 4;
             CB_TEAM_FOR(w, items, tm) {
                 int q = w & 3, g = w >> 2;
-                int blk = g / ngroups, grp = g - blk * ngroups;
-                Cpx *F = buf + blk * nfft + grp * 8 + q;
+                Cpx *F = buf + g * 8 + q;
                 Cpx a = F[0], b = F[4], t;
                 if (q == 0) t = b;
                 else if (q == 1) { t.r = smul(wadd(b.r, b.i), 23170); t.i = smul(wsub(b.i, b.r), 23170); }
@@ -63,8 +64,7 @@ CB_DEV void fft_inplace(TM tm, Cpx *buf, int s, int nblocks) {
             // kf_bfly4 degenerate (kiss_fft.c:121-141)
             const int items = nblocks * ngroups;
             CB_TEAM_FOR(w, items, tm) {
-                int blk = w / ngroups, grp = w - blk * ngroups;
-                Cpx *F = buf + blk * nfft + grp * 4;
+                Cpx *F = buf + w * 4;
                 Cpx f0 = F[0], f1 = F[1], f2 = F[2], f3 = F[3];
                 Cpx s0 = csub(f0, f2);
                 f0 = cadd(f0, f2);
@@ -83,10 +83,10 @@ CB_DEV void fft_inplace(TM tm, Cpx *buf, int s, int nblocks) {
         } else if (p == 4) {
             // kf_bfly4 (kiss_fft.c:142-179)
             const int items = nblocks * ngroups * m;
+            const unsigned mmag = fastdiv_magic(m);
             CB_TEAM_FOR(w, items, tm) {
-                int j = w % m, g = w / m;
-                int blk = g / ngroups, grp = g - blk * ngroups;
-                Cpx *F = buf + blk * nfft + grp * mm + j;
+                int g = fastdiv(w, mmag), j = w - g * m;
+                Cpx *F = buf + w + g * (mm - m);
                 int r1, i1, r2, i2, r3, i3;
                 tw_load(j * fs, r1, i1);
                 tw_load(2 * j * fs, r2, i2);
@@ -110,10 +110,10 @@ CB_DEV void fft_inplace(TM tm, Cpx *buf, int s, int nblocks) {
         } else if (p == 3) {
             // kf_bfly3 (kiss_fft.c:185-240), epi3.i = -28378
             const int items = nblocks * ngroups * m;
+            const unsigned mmag = fastdiv_magic(m);
             CB_TEAM_FOR(w, items, tm) {
-                int j = w % m, g = w / m;
-                int blk = g / ngroups, grp = g - blk * ngroups;
-                Cpx *F = buf + blk * nfft + grp * mm + j;
+                int g = fastdiv(w, mmag), j = w - g * m;
+                Cpx *F = buf + w + g * (mm - m);
                 int r1, i1, r2, i2;
                 tw_load(j * fs, r1, i1);
                 tw_load(2 * j * fs, r2, i2);
@@ -137,10 +137,10 @@ CB_DEV void fft_inplace(TM tm, Cpx *buf, int s, int nblocks) {
         } else {
             // kf_bfly5 (kiss_fft.c:245-318), ya = (10126,-31164), yb = (-26510,-19261)
             const int items = nblocks * ngroups * m;
+            const unsigned mmag = fastdiv_magic(m);
             CB_TEAM_FOR(w, items, tm) {
-                int u = w % m, g = w / m;
-                int blk = g / ngroups, grp = g - blk * ngroups;
-                Cpx *F = buf + blk * nfft + grp * mm + u;
+                int g = fastdiv(w, mmag), u = w - g * m;
+                Cpx *F = buf + w + g * (mm - m);
                 int r1, i1, r2, i2, r3, i3, r4, i4;
                 tw_load(u * fs, r1, i1);
                 tw_load(2 * u * fs, r2, i2);
@@ -189,9 +189,10 @@ CB_DEV void imdct_compute(TM tm, FreqFn freq, int B, int shift, int *fftbuf) {
     CB_NOUNROLL for (int i = 0, n = kMaxFrame * 2; i < shift; i++) { n >>= 1; trig_off += n; }
     const int16_t *t = kMdctTwiddles + trig_off;
     const int16_t *bitrev = fft_bitrev(shift);
+    const unsigned n4mag = fastdiv_magic(N4), halfmag = fastdiv_magic(N4 >> 1);
     // pre-rotate straight into bit-reversed order (mdct.c:283-303)
     CB_TEAM_FOR(w, B * N4, tm) {
-        int b = w / N4, i = w - b * N4;
+        int b = fastdiv(w, n4mag), i = w - b * N4;
         int x1 = freq(b + (2 * i) * B);
         int x2 = freq(b + (N2 - 1 - 2 * i) * B);
         int t0 = t[i], t1 = t[N4 + i];
@@ -204,9 +205,8 @@ CB_DEV void imdct_compute(TM tm, FreqFn freq, int B, int shift, int *fftbuf) {
     tm.sync();
     fft_inplace(tm, (Cpx *)fftbuf, shift, B);
     // post-rotate from both ends (mdct.c:309-343)
-    CB_TEAM_FOR(w, B * ((N4 + 1) >> 1), tm) {
-        int half = (N4 + 1) >> 1;
-        int b = w / half, i = w - b * half;
+    CB_TEAM_FOR(w, B * (N4 >> 1), tm) {   // N4 is even
+        int b = fastdiv(w, halfmag), i = w - b * (N4 >> 1);
         int *yp0 = fftbuf + b * N2 + 2 * i;
         int *yp1 = fftbuf + b * N2 + N2 - 2 - 2 * i;
         int re = yp0[1], im = yp0[0];
@@ -230,14 +230,16 @@ CB_DEV void imdct_compute(TM tm, FreqFn freq, int B, int shift, int *fftbuf) {
 // Second half of the inverse MDCT: block b produced P_b[k] = fftbuf[b*N2+k], destined for
 // out[b*N2 + overlap/2 + k]; positions [b*N2, b*N2+overlap) get the TDAC mirror (mdct.c:346-362).
 // The blocks' mirror regions are disjoint and each reads only un-mirrored P values (or, for block 0,
-// the tail the previous frame left in out[0..overlap/2)), so the whole output is written in one pass.
+// the tail the previous frame left in out[0..overlap/2)), so the whole output is written in one pass.  When sig is given,
+// the frame's samples out[0..N) are also stored to sig[0..N).
 template <class TM>
-CB_DEV void imdct_assemble(TM tm, int *out, int B, int shift, const int *fftbuf) {
+CB_DEV void imdct_assemble(TM tm, int *out, int B, int shift, const int *fftbuf, int *sig = nullptr) {
     const int N2 = (kMaxFrame * 2 >> shift) >> 1;
     const int N = B * N2;
     const int half = kOverlap >> 1;
+    const unsigned n2mag = fastdiv_magic(N2);
     CB_TEAM_FOR(j, N + half, tm) {
-        int b = j / N2;
+        int b = fastdiv(j, n2mag);
         int r = j - b * N2;
         if (b < B && r < kOverlap) {
             if (r < half) {
@@ -249,12 +251,18 @@ CB_DEV void imdct_assemble(TM tm, int *out, int B, int shift, const int *fftbuf)
                 int hi = wadd(smul(x2, kWindow120[i]), smul(x1, kWindow120[kOverlap - 1 - i]));
                 out[b * N2 + i] = lo;
                 out[b * N2 + kOverlap - 1 - i] = hi;
+                if (sig) {
+                    sig[b * N2 + i] = lo;
+                    sig[b * N2 + kOverlap - 1 - i] = hi;
+                }
             }
         } else {
             // straight copy of P (also the un-mirrored tail [N, N+overlap/2) for the next frame)
             int bb = b < B ? b : B - 1;
             int k = j - bb * N2 - half;
-            out[j] = fftbuf[bb * N2 + k];
+            const int v = fftbuf[bb * N2 + k];
+            out[j] = v;
+            if (sig && j < N) sig[j] = v;
         }
     }
     tm.sync();
